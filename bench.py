@@ -9,6 +9,8 @@ block costs 1 280 (aes_encrypt) + 15 (carry bits of add_scalar) + 128 / blocks P
 rank 0 and replicated with one NCCL broadcast; there is no collective on the per-step path.
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched with torchrun)
+  python bench.py ... --dump-outputs DIR                    also writes the output states of the last timed step
+                                                            as .npy files, to compare two builds output for output
   python bench.py --impl reference ...                      CPU arm: the oracle port of the reference's
                                                             CPU path on all host threads (rank 0 only)
 """
@@ -147,13 +149,47 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import aes_clear  # noqa: E402
 
 
-def numpy_decrypt_bytes(ct, glwe_sk):
-    """decrypt_without_padding on the host: ct [..][8][lw] uint64, bit j of a byte in LWE j (client.rs:154)"""
+def numpy_phases(ct, glwe_sk):
+    """b - <a, s> (message + noise) of every LWE of ct [..][lw] uint64, as uint64"""
     ct = ct.reshape(-1, ct.shape[-1])
     with np.errstate(over="ignore"):
-        ph = ct[:, -1] - (ct[:, :-1] * glwe_sk).sum(axis=1, dtype=np.uint64)
-        bits = ((ph + np.uint64(1 << 62)) >> np.uint64(63)).astype(np.uint8) & 1
+        return ct[:, -1] - (ct[:, :-1] * glwe_sk).sum(axis=1, dtype=np.uint64)
+
+
+def numpy_decrypt_bytes(ct, glwe_sk):
+    """decrypt_without_padding on the host: ct [..][8][lw] uint64, bit j of a byte in LWE j (client.rs:154)"""
+    with np.errstate(over="ignore"):
+        bits = ((numpy_phases(ct, glwe_sk) + np.uint64(1 << 62)) >> np.uint64(63)).astype(np.uint8) & 1
     return bytes(np.packbits(bits.reshape(-1, 8), axis=1, bitorder="little").ravel())
+
+
+DUMP_LWE_ROWS = 1024          # whole output LWEs written by --dump-outputs: 1024 x 2049 words = 16.8 MB in float64
+DUMP_PHASES_MAX = 1 << 22     # phases written (32 MB in float64); a larger step writes a seeded sample of this many
+
+
+def torus_f64(x):
+    """uint64 torus elements -> float64 in [-0.5, 0.5): x / 2^64 read as signed (the low ~11 bits of a word are rounded)"""
+    return np.asarray(x, dtype=np.uint64).view(np.int64).astype(np.float64) * 2.0 ** -64
+
+
+def dump_outputs(path, ct, glwe_sk):
+    """Write the output states of one step, ct [blocks][16][8][lw] uint64, as float64 .npy files under path:
+    ciphertexts.npy  [rows][lw]   a sample of the output LWEs, rows drawn with np.random.default_rng(0), sorted;
+    phases.npy       [blocks][16][8] the phase (message + noise) of every output LWE; past DUMP_PHASES_MAX LWEs,
+                     a flat sample drawn with np.random.default_rng(1), sorted.
+    Both are torus values in [-0.5, 0.5).  The samples depend only on the shape, so runs with the same arguments
+    write the same elements."""
+    os.makedirs(path, exist_ok=True)
+    lwes = ct.reshape(-1, ct.shape[-1])
+    n = lwes.shape[0]
+    rows = np.arange(n) if n <= DUMP_LWE_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_LWE_ROWS, replace=False))
+    np.save(os.path.join(path, "ciphertexts.npy"), torus_f64(lwes[rows]))
+    ph = numpy_phases(lwes, glwe_sk)
+    if n <= DUMP_PHASES_MAX:
+        ph = ph.reshape(ct.shape[:-1])
+    else:
+        ph = ph[np.sort(np.random.default_rng(1).choice(n, DUMP_PHASES_MAX, replace=False))]
+    np.save(os.path.join(path, "phases.npy"), torus_f64(ph))
 
 
 class DevPtrArray:
@@ -256,9 +292,10 @@ def run_gpu(args):
     for w in range(args.warmup):
         first = step(w)
     torch.cuda.synchronize()
-    got = decrypt_states(out)     # every warm-up block is verified (client.rs:147-175)
-    for b in range(B):
-        assert got[16 * b:16 * b + 16] == expected(first + b), f"rank {rank}: block {first + b} differs from FIPS-197"
+    if args.warmup:
+        got = decrypt_states(out)     # every block of the last warm-up step is verified (client.rs:147-175)
+        for b in range(B):
+            assert got[16 * b:16 * b + 16] == expected(first + b), f"rank {rank}: block {first + b} differs from FIPS-197"
     sampler = ClockSampler(local)
     launches0 = eng.launch_count
     barrier()
@@ -272,9 +309,13 @@ def run_gpu(args):
     sampler.stop_flag = True
     ms = e0.elapsed_time(e1)
     launches = eng.launch_count - launches0
-    got = decrypt_states(out)
+    out_host = out.cpu().numpy().view(np.uint64).reshape(B, 16, 8, lw)
+    got = numpy_decrypt_bytes(out_host, glwe_sk)
     for b in range(B):
         assert got[16 * b:16 * b + 16] == expected(first + b), f"rank {rank}: block {first + b} differs from FIPS-197"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_host, glwe_sk)
+    del out_host
     first_device = first
     t = torch.tensor([ms, float(launches)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -464,7 +505,12 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE config 1-4 measurements (rank 0)")
     ap.add_argument("--total-blocks", type=int, default=0, help="strong scaling (BASELINE config 5): this many blocks per step split over the GPUs")
     ap.add_argument("--warmup-ref", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output states of the last one (rank 0's blocks) as float64 .npy files "
+                         "under DIR: ciphertexts.npy (a fixed sample of the output LWEs) and phases.npy (message + noise of each)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:
