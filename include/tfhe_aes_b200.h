@@ -85,6 +85,8 @@ int tfa_measure_fp64_peak(tfa_ctx *ctx, double *tflops);   /* max of the two bel
 int tfa_measure_fp64_peaks(tfa_ctx *ctx, double *dfma_tflops, double *dmma_tflops); /* FP64 pipe: DFMA and mma.sync.m8n8k4.f64 microbenchmarks */
 /* number of kernels this library launched on the context since creation (bench.py's gpu_launches) */
 uint64_t tfa_ctx_launch_count(const tfa_ctx *ctx);
+/* LWE ciphertexts blind-rotated (programmable bootstraps, circuit-bootstrap ones included) on the context since creation */
+uint64_t tfa_ctx_pbs_count(const tfa_ctx *ctx);
 
 /* ---- sbox module --------------------------------------------------------------------------------- */
 /* gen_lut (gen_lut.rs:9-42): table[v] = f(v) for v < 2^(nb_block*log2(msg*carry));
@@ -128,6 +130,26 @@ int tfa_aes_ctr(tfa_ctx *ctx, const uint64_t *round_keys, const uint64_t *iv_ct,
  * encryptions of the data.  With one message bit per LWE at 2^63 a clear bit adds bit * 2^63 to the body: no bootstrap. */
 int tfa_xor_clear(tfa_ctx *ctx, uint64_t *states, const uint8_t *data, int nblk);
 int tfa_xor_clear_dev(tfa_ctx *ctx, uint64_t *states, const uint8_t *data_dev, int nblk);
+/* AES-CTR with a PUBLIC initial counter block (only the AES key is encrypted, as in AES-CTR transciphering, where the IV travels in
+ * the clear), for nstreams independent streams that share the context's FHE keys.  Output block b of stream s =
+ * Enc( AES_K_s(iv_s + first_s + b mod 2^128) XOR data_s[b] ), in stream order: out [sum of nblk][16][8][lw].  rounds = 10 / 12 / 14
+ * (AES-128 / 192 / 256); round_keys of each stream [rounds + 1][16][8][lw] (tfa_aes_key_expansion[_ex] output).  data NULL: the bare
+ * keystream.  No counter add is evaluated; the first two rounds are evaluated once per run of counters that agree on bytes 0..14
+ * (at most 256 blocks): 8 * (27 * runs + (16 * (rounds - 2) + 5) * blocks) PBS in all, 133 byte-WoPBS per AES-128 block instead of 160.
+ * Errors: TFA_ERR_PARAM for nstreams < 1, an nblk < 1, a NULL round_keys, more than INT_MAX / 16 blocks in all or another rounds;
+ * TFA_ERR_STATE without keys; TFA_ERR_UNSUPPORTED unless blocks carry one bit (message_modulus * carry_modulus = 2). */
+typedef struct tfa_ctr_stream {
+    const uint64_t *round_keys;
+    const uint8_t *data;          /* [nblk][16] or NULL */
+    uint64_t first_lo, first_hi;
+    uint8_t iv[16];               /* AES byte order, byte 0 = most significant */
+    int32_t nblk;
+    int32_t _pad;
+} tfa_ctr_stream;                 /* 56 bytes, no implicit padding */
+/* host pointers; every distinct round-key buffer is copied once; synchronises before returning */
+int tfa_aes_ctr_public_iv(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, uint64_t *out);
+/* streams: host array whose round_keys and data are device pointers; out: device; asynchronous on the context stream */
+int tfa_aes_ctr_public_iv_dev(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, uint64_t *out);
 /* one AES round on nblk states (BASELINE config 2): 16*nblk many_sbox + ShiftRows/MixColumns + AddRoundKey */
 int tfa_aes_round(tfa_ctx *ctx, const uint64_t *round_key, uint64_t *states, int nblk);
 /* linear layers alone (server.rs:278-282, mix_columns.rs:4, inv_mix_columns.rs:4, shift_rows.rs:5, inv_shift_rows.rs:5) */

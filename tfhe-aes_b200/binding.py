@@ -43,6 +43,23 @@ def param_test2():
     return Params(24, 1, 512, 8, 5, 2, 6, 12, 3, 15, 1, 4, 1, 0, 2.0 ** -24, 2.0 ** -50, 2.0 ** -50)
 
 
+class TfaCtrStream(C.Structure):
+    """tfa_ctr_stream: one public-IV AES-CTR stream (include/tfhe_aes_b200.h)."""
+    _fields_ = [("round_keys", C.c_void_p), ("data", C.c_void_p), ("first_lo", C.c_uint64), ("first_hi", C.c_uint64),
+                ("iv", C.c_uint8 * 16), ("nblk", C.c_int32), ("_pad", C.c_int32)]
+
+
+assert C.sizeof(TfaCtrStream) == 56
+
+
+def _ctr_stream(rk_ptr, iv, first, nblk, data_ptr):
+    iv = iv.to_bytes(16, "big") if isinstance(iv, int) else bytes(iv)
+    if len(iv) != 16:
+        raise ValueError("iv must be an int or 16 bytes")
+    first %= 2 ** 128
+    return TfaCtrStream(rk_ptr, data_ptr, first & (2 ** 64 - 1), first >> 64, (C.c_uint8 * 16)(*iv), nblk, 0)
+
+
 _lib = None
 
 _SIGS = {
@@ -72,6 +89,8 @@ _SIGS = {
     "tfa_xor_clear": [C.c_void_p, C.c_void_p, C.c_char_p, C.c_int],
     "tfa_xor_clear_dev": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
     "tfa_aes_ctr_dev": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p],
+    "tfa_aes_ctr_public_iv": [C.c_void_p, C.POINTER(TfaCtrStream), C.c_int, C.c_int, C.c_void_p],
+    "tfa_aes_ctr_public_iv_dev": [C.c_void_p, C.POINTER(TfaCtrStream), C.c_int, C.c_int, C.c_void_p],
     "tfa_add_round_key": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
     "tfa_mix_columns": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
     "tfa_inv_mix_columns": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
@@ -113,6 +132,8 @@ def load_library():
         lib.tfa_last_error.argtypes = [C.c_void_p]
         lib.tfa_ctx_launch_count.restype = C.c_uint64
         lib.tfa_ctx_launch_count.argtypes = [C.c_void_p]
+        lib.tfa_ctx_pbs_count.restype = C.c_uint64
+        lib.tfa_ctx_pbs_count.argtypes = [C.c_void_p]
         lib.tfa_ctx_destroy.argtypes = [C.c_void_p]
         lib.tfa_ctx_destroy.restype = None
         for name in ("tfa_ctx_alloc_keys", "tfa_ctx_keys_ready", "tfa_ctx_synchronize"):
@@ -230,6 +251,11 @@ class Engine:
     def launch_count(self):
         return int(self.lib.tfa_ctx_launch_count(self.h))
 
+    @property
+    def pbs_count(self):
+        """LWE ciphertexts blind-rotated on this context since creation"""
+        return int(self.lib.tfa_ctx_pbs_count(self.h))
+
     def synchronize(self):
         self._ck(self.lib.tfa_ctx_synchronize(self.h))
 
@@ -266,6 +292,12 @@ class Engine:
 
     def aes_ctr_dev(self, rk_ptr, iv_ptr, first, nblk, out_ptr):
         self._ck(self.lib.tfa_aes_ctr_dev(self.h, C.c_void_p(rk_ptr), C.c_void_p(iv_ptr), first & (2 ** 64 - 1), first >> 64, nblk, C.c_void_p(out_ptr)))
+
+    def aes_ctr_public_iv_dev(self, streams, out_ptr, rounds=10):
+        """streams: list of (round_keys device pointer, iv (int or 16 bytes), first, nblk, data device pointer or None);
+        out_ptr: device [total][16][8][lw].  Asynchronous on the context stream."""
+        arr = (TfaCtrStream * len(streams))(*[_ctr_stream(rk, iv, first, nblk, data) for rk, iv, first, nblk, data in streams])
+        self._ck(self.lib.tfa_aes_ctr_public_iv_dev(self.h, arr, len(streams), rounds, C.c_void_p(out_ptr) if out_ptr else None))
 
     def aes_encrypt_dev(self, rk_ptr, st_ptr, nblk):
         self._ck(self.lib.tfa_aes_encrypt_dev(self.h, C.c_void_p(rk_ptr), C.c_void_p(st_ptr), nblk))
@@ -408,6 +440,30 @@ class Engine:
         iv_ct = np.ascontiguousarray(iv_ct, dtype=np.uint64)
         out = np.zeros((nblk, 16, 8, self.lw), dtype=np.uint64)
         self._ck(self.lib.tfa_aes_ctr(self.h, _p(rk), _p(iv_ct), first & (2 ** 64 - 1), first >> 64, nblk, _p(out)))
+        return out
+
+    def aes_ctr_public_iv(self, streams, rounds=10):
+        """AES-CTR with public IVs, many streams in one call.  streams: list of (round_keys [rounds+1][16][8][lw], iv (int or
+        16 bytes, AES byte order), first, nblk, data (16 * nblk bytes) or None).  Returns [total][16][8][lw]: block b of a stream
+        encrypts AES(iv + first + b) XOR data[b], streams in order."""
+        keep, rks = [], {}
+        for rk, _, _, _, _ in streams:   # one array per distinct round-key object: the library uploads each pointer once
+            if rk is not None and id(rk) not in rks:
+                rks[id(rk)] = np.ascontiguousarray(rk, dtype=np.uint64)
+        structs = []
+        for rk, iv, first, nblk, data in streams:
+            d = None
+            if data is not None:
+                d = np.frombuffer(bytes(data), dtype=np.uint8).copy()
+                if len(d) != 16 * nblk:
+                    raise ValueError("data must hold 16 bytes per block")
+                keep.append(d)
+            structs.append(_ctr_stream(_p(rks[id(rk)]) if rk is not None else None, iv, first, nblk, _p(d)))
+        total = sum(max(int(s.nblk), 0) for s in structs)
+        # an out-of-range total is left to the library to reject (TFA_ERR_PARAM) without allocating for it
+        out = np.zeros((total, 16, 8, self.lw), dtype=np.uint64) if 0 < total < 2 ** 27 else None
+        arr = (TfaCtrStream * len(structs))(*structs)
+        self._ck(self.lib.tfa_aes_ctr_public_iv(self.h, arr, len(structs), rounds, _p(out)))
         return out
 
     def xor_clear(self, states, data: bytes):

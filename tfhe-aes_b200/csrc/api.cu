@@ -2,7 +2,9 @@
 // device stages of engine.cu.  Orchestration follows server.rs / sbox.rs line by line; the per-byte
 // loops of the reference (server.rs:47-50, 59-61, 76-78, 88-91, 100-102) become one batched pass
 // over all bytes of all resident blocks.
+#include <algorithm>
 #include <chrono>
+#include <climits>
 #include <condition_variable>
 #include <cstring>
 #include <mutex>
@@ -190,17 +192,19 @@ static int lin_add_round_key(tfa_ctx *ctx, u64 *state, const u64 *rk, int nblk) 
     }
     return dev_lwe_sum(ctx, v, (int)bw);
 }
-// state[b][4c+row] = MixColumns(ShiftRows(mul))[..] (+ rk)                    (mix_columns.rs:4-78)
-static int lin_mix_columns(tfa_ctx *ctx, const u64 *mul, u64 *state, const u64 *rk, int nblk) {
+// the same round key for each of nblk blocks
+static std::vector<const u64 *> same_rk(const u64 *rk, int nblk) { return std::vector<const u64 *>((size_t)nblk, rk); }
+// state[b][4c+row] = MixColumns(ShiftRows(mul))[..] (+ rk[b])                 (mix_columns.rs:4-78)
+// MIX_PICK[row][j] = which of {S,2S,3S} of shifted byte j of the column (mix_columns.rs:36-75)
+static const int MIX_PICK[4][4] = {{1, 2, 0, 0}, {0, 1, 2, 0}, {0, 0, 1, 2}, {2, 0, 0, 1}};
+static int lin_mix_columns(tfa_ctx *ctx, const u64 *mul, u64 *state, const u64 *const *rk, int nblk) {
     const size_t bw = ctx->byte_words();
     std::vector<SumEntry> v;
-    // picks[row][j] = which of {S,2S,3S} of shifted byte j of the column (mix_columns.rs:36-75)
-    static const int pick[4][4] = {{1, 2, 0, 0}, {0, 1, 2, 0}, {0, 0, 1, 2}, {2, 0, 0, 1}};
     for (int b = 0; b < nblk; b++) for (int col = 0; col < 4; col++) for (int row = 0; row < 4; row++) {
         SumEntry e{};
         e.dst = state + ((size_t)b * 16 + 4 * col + row) * bw;
-        for (int j = 0; j < 4; j++) e.src[e.nsrc++] = mul + (((size_t)b * 16 + sr(4 * col + j)) * 3 + pick[row][j]) * bw;
-        if (rk) e.src[e.nsrc++] = rk + (size_t)(4 * col + row) * bw;
+        for (int j = 0; j < 4; j++) e.src[e.nsrc++] = mul + (((size_t)b * 16 + sr(4 * col + j)) * 3 + MIX_PICK[row][j]) * bw;
+        if (rk) e.src[e.nsrc++] = rk[b] + (size_t)(4 * col + row) * bw;
         v.push_back(e);
     }
     return dev_lwe_sum(ctx, v, (int)bw);
@@ -240,7 +244,8 @@ static size_t aes_scratch(const tfa_ctx *ctx, int nblk, int L) {
     const size_t w = (size_t)nblk * 16 * ctx->byte_words() * 8;
     return many_wopbs_scratch(ctx, nblk * 16, nb, L * nb, tfa_lut_size(&ctx->p, nb)) * 2 + w * (L + 2) + (size_t)nblk * 16 * sizeof(SumEntry) * 4;
 }
-static int aes_round_nolock(tfa_ctx *ctx, const u64 *rk_round, u64 *state, int nblk, u64 *mul) {
+// rk_round[b]: round key of block b
+static int aes_round_nolock(tfa_ctx *ctx, const u64 *const *rk_round, u64 *state, int nblk, u64 *mul) {
     RC(sbox_like_dev(ctx, state, nblk * 16, 1, mul));                      // server.rs:47-50 (many_sbox)
     return lin_mix_columns(ctx, mul, state, rk_round, nblk);               // server.rs:53-55
 }
@@ -252,7 +257,7 @@ static int aes_encrypt_nolock(tfa_ctx *ctx, const u64 *rk, u64 *state, int nblk,
     RC(lin_add_round_key(ctx, state, rk, nblk));                           // server.rs:42
     for (int round = 1; round < nr; round++) {
         ctx->ws_off = mark;
-        RC(aes_round_nolock(ctx, rk + (size_t)round * rkw, state, nblk, mul));
+        RC(aes_round_nolock(ctx, same_rk(rk + (size_t)round * rkw, nblk).data(), state, nblk, mul));
     }
     ctx->ws_off = mark;
     RC(sbox_like_dev(ctx, state, nblk * 16, 0, mul));                      // server.rs:59-61
@@ -437,7 +442,7 @@ extern "C" int tfa_aes_round_dev(tfa_ctx *ctx, const uint64_t *rk_round, uint64_
     RC(require_keys(ctx));
     RC(ws_reserve(ctx, aes_scratch(ctx, nblk, 3)));
     WSB(mul, u64, (size_t)nblk * 16 * 3 * ctx->byte_words());
-    return aes_round_nolock(ctx, rk_round, states, nblk, mul);
+    return aes_round_nolock(ctx, same_rk(rk_round, nblk).data(), states, nblk, mul);
 }
 extern "C" int tfa_add_scalar_dev(tfa_ctx *ctx, uint64_t *states, const uint64_t *ctr_dev, int nblk) {
     Guard g(ctx);
@@ -480,6 +485,158 @@ extern "C" int tfa_aes_ctr_dev(tfa_ctx *ctx, const uint64_t *rk, const uint64_t 
     size_t a = aes_scratch(ctx, nblk, 3), b = add_scalar_scratch(ctx, nblk);
     RC(ws_reserve(ctx, (a > b ? a : b) + (size_t)nblk * 16));
     return aes_ctr_nolock(ctx, rk, iv_ct, first_lo, first_hi, nblk, out);
+}
+
+// ---- AES-CTR with a public IV ------------------------------------------------------------------------------------
+// The counter blocks are known in the clear, so no counter add is evaluated: round 0 is the round key XOR a clear block (body
+// words only, lwe_sum_xor).  Consecutive counters that agree on bytes 0..14 (a run, at most 256 blocks) differ in byte 15 alone:
+//   round 1: only S-box input 15 differs per block; ShiftRows moves it to column 0, so after MixColumns + AddRoundKey bytes 0..3
+//            differ per block and bytes 4..15 are the same ciphertexts for the whole run;
+//   round 2: S-boxes 0..3 per block, 4..15 per run; every output column mixes exactly one per-block product with three per-run
+//            ones, so from round 3 on all 16 bytes are per block.
+// S-box evaluations: 15 + 12 = 27 per run and 1 + 4 + 16 (Nr - 2) per block (133 for AES-128 instead of 160 + the counter add).
+struct CtrPlan {
+    int G = 0, B = 0;                  // runs, blocks
+    std::vector<int> blk_run, blk_stream, blk_pos;   // run, stream and position in its stream of each block
+    std::vector<uint8_t> blk_low;      // byte 15 of the counter block of each block
+    std::vector<int> run_stream;
+    std::vector<uint8_t> run_high;     // [G][15]: bytes 0..14 of the counter blocks of each run
+};
+static int plan_public_ctr(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, CtrPlan &p) {
+    if (!streams || nstreams < 1) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_public_iv: nstreams must be >= 1");
+    if (rounds != 10 && rounds != 12 && rounds != 14) return ctx->fail(TFA_ERR_PARAM, "rounds must be 10, 12 or 14");
+    long long total = 0;
+    for (int s = 0; s < nstreams; s++) {
+        if (streams[s].nblk < 1 || !streams[s].round_keys) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_public_iv: every stream needs nblk >= 1 and round keys");
+        total += streams[s].nblk;
+    }
+    // 16 encrypted bytes per block are indexed with int in the S-box batches
+    if (total > INT_MAX / 16) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_public_iv: too many blocks in one call");
+    typedef unsigned __int128 u128;
+    p.B = (int)total;
+    for (int s = 0; s < nstreams; s++) {
+        u128 c = 0;
+        for (int i = 0; i < 16; i++) c = (c << 8) | streams[s].iv[i];
+        c += ((u128)streams[s].first_hi << 64) | streams[s].first_lo;          // wraps mod 2^128
+        for (int b = 0; b < streams[s].nblk; b++) {
+            const u128 ctr = c + (u128)b;
+            const uint8_t low = (uint8_t)ctr;
+            if (b == 0 || low == 0) {                                          // a new run, also at the wrap to 0
+                p.run_stream.push_back(s);
+                for (int i = 0; i < 15; i++) p.run_high.push_back((uint8_t)(ctr >> (8 * (15 - i))));
+                p.G++;
+            }
+            p.blk_run.push_back(p.G - 1); p.blk_stream.push_back(s); p.blk_pos.push_back(b); p.blk_low.push_back(low);
+        }
+    }
+    return TFA_OK;
+}
+static size_t ctr_public_scratch(const tfa_ctx *ctx, int G, int B) {
+    const int nb = nblocks_per_byte(ctx);
+    const size_t n1 = (size_t)15 * G + B, n2 = (size_t)12 * G + (size_t)4 * B, n3 = (size_t)16 * B, bw8 = ctx->byte_words() * 8;
+    const size_t nmax = std::max(n1, std::max(n2, n3));
+    return many_wopbs_scratch(ctx, (int)nmax, nb, 3 * nb, tfa_lut_size(&ctx->p, nb)) * 2 + (n1 + n2) * 4 * bw8 + n3 * 3 * bw8 +
+           nmax * sizeof(SumXorEntry) * 2;
+}
+// streams[s].round_keys / data: device pointers; out [B][16][8][lw] device, also the state of rounds 2 .. nr-1
+static int aes_ctr_public_nolock(tfa_ctx *ctx, const tfa_ctr_stream *streams, const CtrPlan &p, int nr, u64 *out) {
+    const size_t bw = ctx->byte_words(), rkw = 16 * bw;
+    const int G = p.G, B = p.B, n1 = 15 * G + B, n2 = 12 * G + 4 * B;
+    WSB(x1, u64, (size_t)n1 * bw);                // round-1 S-box inputs: [G][15] per run, then [B] (byte 15)
+    WSB(m1, u64, (size_t)n1 * 3 * bw);
+    WSB(x2, u64, (size_t)n2 * bw);                // round-2 S-box inputs: [G][12] per run (bytes 4..15), then [B][4] (bytes 0..3)
+    WSB(m2, u64, (size_t)n2 * 3 * bw);
+    WSB(mul, u64, (size_t)B * 16 * 3 * bw);
+    const size_t mark = ctx->ws_off;
+    auto rk_of = [&](int stream, int round, int byte) { return streams[stream].round_keys + (size_t)round * rkw + (size_t)byte * bw; };
+    // (1) AddRoundKey with the clear counter block, then the round-1 S-boxes of all runs and blocks in one batch
+    {
+        std::vector<SumXorEntry> v;
+        v.reserve(n1);
+        for (int g = 0; g < G; g++) for (int i = 0; i < 15; i++) {
+            SumXorEntry e{};
+            e.dst = x1 + ((size_t)15 * g + i) * bw; e.src[e.nsrc++] = rk_of(p.run_stream[g], 0, i); e.clear = p.run_high[(size_t)15 * g + i];
+            v.push_back(e);
+        }
+        for (int b = 0; b < B; b++) {
+            SumXorEntry e{};
+            e.dst = x1 + ((size_t)15 * G + b) * bw; e.src[e.nsrc++] = rk_of(p.blk_stream[b], 0, 15); e.clear = p.blk_low[b];
+            v.push_back(e);
+        }
+        RC(dev_lwe_sum_xor(ctx, v));
+        RC(sbox_like_dev(ctx, x1, n1, 1, m1));
+    }
+    // (2) round-1 MixColumns + AddRoundKey: columns 1..3 once per run, column 0 per block; then the round-2 S-boxes
+    ctx->ws_off = mark;
+    {
+        // {S,2S,3S} of round-1 state byte i: per block for i = 15, per run otherwise
+        auto s1 = [&](int g, int b, int i, int k) { return m1 + ((i == 15 ? (size_t)15 * G + b : (size_t)15 * g + i) * 3 + k) * bw; };
+        std::vector<SumEntry> v;
+        v.reserve(n2);
+        for (int g = 0; g < G; g++) for (int col = 1; col < 4; col++) for (int row = 0; row < 4; row++) {
+            SumEntry e{};
+            e.dst = x2 + ((size_t)12 * g + 4 * col + row - 4) * bw;
+            for (int j = 0; j < 4; j++) e.src[e.nsrc++] = s1(g, -1, sr(4 * col + j), MIX_PICK[row][j]);   // sr(4 col + j) != 15 for col > 0
+            e.src[e.nsrc++] = rk_of(p.run_stream[g], 1, 4 * col + row);
+            v.push_back(e);
+        }
+        for (int b = 0; b < B; b++) for (int row = 0; row < 4; row++) {
+            SumEntry e{};
+            e.dst = x2 + ((size_t)12 * G + (size_t)4 * b + row) * bw;
+            for (int j = 0; j < 4; j++) e.src[e.nsrc++] = s1(p.blk_run[b], b, sr(j), MIX_PICK[row][j]);
+            e.src[e.nsrc++] = rk_of(p.blk_stream[b], 1, row);
+            v.push_back(e);
+        }
+        RC(dev_lwe_sum(ctx, v, (int)bw));
+        RC(sbox_like_dev(ctx, x2, n2, 1, m2));
+    }
+    // (3) round-2 MixColumns + AddRoundKey: the full per-block state
+    ctx->ws_off = mark;
+    {
+        auto s2 = [&](int g, int b, int i, int k) { return m2 + ((i < 4 ? (size_t)12 * G + (size_t)4 * b + i : (size_t)12 * g + i - 4) * 3 + k) * bw; };
+        std::vector<SumEntry> v;
+        v.reserve((size_t)16 * B);
+        for (int b = 0; b < B; b++) for (int col = 0; col < 4; col++) for (int row = 0; row < 4; row++) {
+            SumEntry e{};
+            e.dst = out + ((size_t)b * 16 + 4 * col + row) * bw;
+            for (int j = 0; j < 4; j++) e.src[e.nsrc++] = s2(p.blk_run[b], b, sr(4 * col + j), MIX_PICK[row][j]);
+            e.src[e.nsrc++] = rk_of(p.blk_stream[b], 2, 4 * col + row);
+            v.push_back(e);
+        }
+        RC(dev_lwe_sum(ctx, v, (int)bw));
+    }
+    // (4) rounds 3 .. nr-1 as aes_encrypt_nolock, with the round key of each block's stream
+    std::vector<const u64 *> rkb((size_t)B);
+    for (int round = 3; round < nr; round++) {
+        ctx->ws_off = mark;
+        for (int b = 0; b < B; b++) rkb[b] = rk_of(p.blk_stream[b], round, 0);
+        RC(aes_round_nolock(ctx, rkb.data(), out, B, mul));
+    }
+    // (5) final round: S-box, then ShiftRows + AddRoundKey + XOR with the clear data in one pass
+    ctx->ws_off = mark;
+    RC(sbox_like_dev(ctx, out, B * 16, 0, mul));
+    std::vector<SumXorEntry> v;
+    v.reserve((size_t)16 * B);
+    for (int b = 0; b < B; b++) for (int i = 0; i < 16; i++) {
+        const tfa_ctr_stream &st = streams[p.blk_stream[b]];
+        SumXorEntry e{};
+        e.dst = out + ((size_t)b * 16 + i) * bw;
+        e.src[e.nsrc++] = mul + ((size_t)b * 16 + sr(i)) * bw;
+        e.src[e.nsrc++] = rk_of(p.blk_stream[b], nr, i);
+        e.clear_src = st.data ? st.data + (size_t)p.blk_pos[b] * 16 + i : nullptr;
+        v.push_back(e);
+    }
+    return dev_lwe_sum_xor(ctx, v);
+}
+extern "C" int tfa_aes_ctr_public_iv_dev(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, uint64_t *out) {
+    Guard g(ctx);
+    CtrPlan p;
+    RC(plan_public_ctr(ctx, streams, nstreams, rounds, p));
+    if (!out) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_public_iv: null output");
+    RC(require_keys(ctx));
+    if (nblocks_per_byte(ctx) != 8) return ctx->fail(TFA_ERR_UNSUPPORTED, "aes_ctr_public_iv needs 1-bit blocks (client.rs:53-54)");
+    RC(ws_reserve(ctx, ctr_public_scratch(ctx, p.G, p.B)));
+    return aes_ctr_public_nolock(ctx, streams, p, rounds, out);
 }
 
 // ---- host-pointer entry points ---------------------------------------------------------------------
@@ -591,7 +748,7 @@ extern "C" int tfa_aes_round(tfa_ctx *ctx, const uint64_t *round_key, uint64_t *
     RC(ws_reserve(ctx, aes_scratch(ctx, nblk, 3) + (sw + 16 * bw) * 8));
     WSB(d_rk, u64, 16 * bw); WSB(d_st, u64, sw); WSB(mul, u64, sw * 3);
     H2D(d_rk, round_key, 16 * bw); H2D(d_st, states, sw);
-    RC(aes_round_nolock(ctx, d_rk, d_st, nblk, mul));
+    RC(aes_round_nolock(ctx, same_rk(d_rk, nblk).data(), d_st, nblk, mul));
     D2H(states, d_st, sw);
     SYNC();
     return TFA_OK;
@@ -651,6 +808,41 @@ extern "C" int tfa_aes_ctr(tfa_ctx *ctx, const uint64_t *round_keys, const uint6
     WSB(d_rk, u64, rkw); WSB(d_iv, u64, 16 * bw); WSB(d_out, u64, sw);
     H2D(d_rk, round_keys, rkw); H2D(d_iv, iv_ct, 16 * bw);
     RC(aes_ctr_nolock(ctx, d_rk, d_iv, first_lo, first_hi, nblk, d_out));
+    D2H(out, d_out, sw);
+    SYNC();
+    return TFA_OK;
+}
+extern "C" int tfa_aes_ctr_public_iv(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, uint64_t *out) {
+    Guard g(ctx);
+    CtrPlan p;
+    RC(plan_public_ctr(ctx, streams, nstreams, rounds, p));
+    if (!out) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_public_iv: null output");
+    RC(require_keys(ctx));
+    if (nblocks_per_byte(ctx) != 8) return ctx->fail(TFA_ERR_UNSUPPORTED, "aes_ctr_public_iv needs 1-bit blocks (client.rs:53-54)");
+    const size_t bw = ctx->byte_words(), rkw = (size_t)(rounds + 1) * 16 * bw, sw = (size_t)p.B * 16 * bw;
+    std::vector<const u64 *> keys;                       // distinct round-key buffers: streams under one AES key upload it once
+    for (int s = 0; s < nstreams; s++)
+        if (std::find(keys.begin(), keys.end(), streams[s].round_keys) == keys.end()) keys.push_back(streams[s].round_keys);
+    RC(ws_reserve(ctx, ctr_public_scratch(ctx, p.G, p.B) + (keys.size() * rkw + sw) * 8 + (size_t)p.B * 16 + 256 * (keys.size() + 2)));
+    WSB(d_out, u64, sw);
+    WSB(d_data, uint8_t, (size_t)p.B * 16);
+    std::vector<u64 *> d_keys;
+    for (auto k : keys) {
+        WSB(d, u64, rkw);
+        H2D(d, k, rkw);
+        d_keys.push_back(d);
+    }
+    std::vector<tfa_ctr_stream> dev(streams, streams + nstreams);
+    size_t off = 0;
+    for (int s = 0; s < nstreams; s++) {
+        dev[s].round_keys = d_keys[std::find(keys.begin(), keys.end(), streams[s].round_keys) - keys.begin()];
+        if (streams[s].data) {
+            CU(cudaMemcpyAsync(d_data + off, streams[s].data, (size_t)streams[s].nblk * 16, cudaMemcpyHostToDevice, ctx->stream));
+            dev[s].data = d_data + off;
+        }
+        off += (size_t)streams[s].nblk * 16;
+    }
+    RC(aes_ctr_public_nolock(ctx, dev.data(), p, rounds, d_out));
     D2H(out, d_out, sw);
     SYNC();
     return TFA_OK;

@@ -81,6 +81,7 @@ extern "C" int tfa_ctx_create(const tfa_params *p, int device, void *stream, tfa
     ctx->sm_count = 148;
     cudaDeviceGetAttribute(&ctx->sm_count, cudaDevAttrMultiProcessorCount, device);
     ctx->launches = 0;
+    ctx->pbs_count = 0;
     ctx->profiling = false;
     ctx->pbs_schedule = 0;
     ctx->own_stream = (stream == nullptr);
@@ -129,6 +130,7 @@ extern "C" int tfa_ctx_set_pbs_schedule(tfa_ctx *ctx, int schedule) {
     return TFA_OK;
 }
 extern "C" uint64_t tfa_ctx_launch_count(const tfa_ctx *ctx) { return ctx->launches; }
+extern "C" uint64_t tfa_ctx_pbs_count(const tfa_ctx *ctx) { return ctx->pbs_count; }
 
 // ------------------------------------------------------------------------------------------------
 // key preparation
@@ -302,6 +304,7 @@ int dev_pfks(tfa_ctx *ctx, const u64 *in, int count, u64 *out, int out_stride) {
 // SURVEY §9.4(3)
 int dev_pbs(tfa_ctx *ctx, const u64 *in, int count, const u64 *lut, u64 in_scale, u64 pre_add, u64 post_add, u64 *out) {
     StageTimer t(ctx, ST_PBS);
+    ctx->pbs_count += (u64)count;
     PbsArgs a{};
     a.lwe_in = in; a.bsk = ctx->bsk_f; a.tw = ctx->tw; a.lut = lut; a.out = out;
     a.in_scale = in_scale; a.pre_add_body = pre_add; a.post_add = post_add; a.lwe_dim = ctx->n; a.count = count;
@@ -547,16 +550,31 @@ static int pin_stage(tfa_ctx *ctx, size_t bytes, char **out) {
     return TFA_OK;
 }
 
+// the gather list goes through the context's pinned ring: the copy is asynchronous (a pageable source of this size would
+// make the driver synchronise the stream) and does not depend on the lifetime of the host table
+template <typename E>
+static int upload_table(tfa_ctx *ctx, const std::vector<E> &entries, E **out) {
+    WS(d, E, entries.size());
+    char *stage = nullptr;
+    RC(pin_stage(ctx, entries.size() * sizeof(E), &stage));
+    memcpy(stage, entries.data(), entries.size() * sizeof(E));
+    CU(cudaMemcpyAsync(d, stage, entries.size() * sizeof(E), cudaMemcpyHostToDevice, ctx->stream));
+    *out = d;
+    return TFA_OK;
+}
 int dev_lwe_sum(tfa_ctx *ctx, const std::vector<SumEntry> &entries, int unit_words) {
     StageTimer t(ctx, ST_LINEAR);
-    WS(d, SumEntry, entries.size());
-    // the gather list goes through the context's pinned ring: the copy is asynchronous (a pageable source of this size would
-    // make the driver synchronise the stream) and does not depend on the lifetime of `entries`
-    char *stage = nullptr;
-    RC(pin_stage(ctx, entries.size() * sizeof(SumEntry), &stage));
-    memcpy(stage, entries.data(), entries.size() * sizeof(SumEntry));
-    CU(cudaMemcpyAsync(d, stage, entries.size() * sizeof(SumEntry), cudaMemcpyHostToDevice, ctx->stream));
+    SumEntry *d = nullptr;
+    RC(upload_table(ctx, entries, &d));
     CU(launch_lwe_sum(d, (int)entries.size(), unit_words, ctx->stream));
+    ctx->launches++;
+    return TFA_OK;
+}
+int dev_lwe_sum_xor(tfa_ctx *ctx, const std::vector<SumXorEntry> &entries) {
+    StageTimer t(ctx, ST_LINEAR);
+    SumXorEntry *d = nullptr;
+    RC(upload_table(ctx, entries, &d));
+    CU(launch_lwe_sum_xor(d, (int)entries.size(), ctx->lw, ctx->stream));
     ctx->launches++;
     return TFA_OK;
 }

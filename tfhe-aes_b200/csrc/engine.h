@@ -19,6 +19,7 @@ struct tfa_ctx {
     std::string err;
     std::mutex mu;
     u64 launches;
+    u64 pbs_count;         // LWE ciphertexts blind-rotated since creation (tfa_ctx_pbs_count)
 
     // prepared keys (device)
     double2 *bsk_f;        // [n][pbs_level][k+1][k+1][256]
@@ -126,5 +127,6 @@ int dev_many_wopbs(tfa_ctx *ctx, const u64 *ct_in, int nct, int nblocks, const u
                    size_t lut_out_stride, int nouts, int lut_size, u64 *out);
 size_t many_wopbs_scratch(const tfa_ctx *ctx, int nct, int nblocks, int nouts, int lut_size);
 int dev_lwe_sum(tfa_ctx *ctx, const std::vector<SumEntry> &entries, int unit_words);
+int dev_lwe_sum_xor(tfa_ctx *ctx, const std::vector<SumXorEntry> &entries);  // one encrypted byte per entry
 int require_keys(tfa_ctx *ctx);
 const u64 *cached_lut(tfa_ctx *ctx, int which);  // device pointer, see lut_cache

@@ -1,6 +1,7 @@
 // int_kernels.cu — elementwise integer (u64 wrapping) kernels of the WoPBS chain (sm_100a):
 //   lwe_sum            fused ShiftRows / MixColumns / AddRoundKey additions (K7; server.rs:278-282,
 //                      mix_columns.rs:4-78, inv_mix_columns.rs:4-58)
+//   lwe_sum_xor        the same plus a clear byte XORed in (public-IV CTR: counter bytes, data bytes)
 //   gemv_init          output initialisation of the keyswitch / PFKS products (imma_kernels.cu)
 //   helpers of the general extract_bits loop, CMux-tree leaves, add_scalar LUT generation.
 #include "kernels.h"
@@ -36,6 +37,25 @@ __global__ void lwe_sum_kernel(const SumEntry *__restrict__ entries, int unit_wo
 cudaError_t launch_lwe_sum(const SumEntry *entries, int nentries, int unit_words, cudaStream_t s) {
     dim3 grid((unit_words + 1023) / 1024, nentries);
     lwe_sum_kernel<<<grid, 256, 0, s>>>(entries, unit_words);
+    return cudaGetLastError();
+}
+// the same over one encrypted byte (8 LWEs of lw words) per entry, plus the clear byte on the 8 body words: with one message
+// bit per LWE at 2^63, adding the encoded bit is the XOR (no bootstrap, no added noise)
+__global__ void lwe_sum_xor_kernel(const SumXorEntry *__restrict__ entries, int lw) {
+    const SumXorEntry e = entries[blockIdx.y];
+    const uint32_t clear = e.clear ^ (e.clear_src ? *e.clear_src : 0u);
+    const int unit_words = 8 * lw;
+    for (int w = blockIdx.x * blockDim.x + threadIdx.x; w < unit_words; w += gridDim.x * blockDim.x) {
+        uint64_t s = e.src[0][w];
+        for (int t = 1; t < e.nsrc; t++) s += e.src[t][w];
+        const uint32_t j = (uint32_t)w / (uint32_t)lw;
+        if ((uint32_t)w - j * (uint32_t)lw == (uint32_t)lw - 1) s += (uint64_t)((clear >> j) & 1) << 63;
+        e.dst[w] = s;
+    }
+}
+cudaError_t launch_lwe_sum_xor(const SumXorEntry *entries, int nentries, int lw, cudaStream_t s) {
+    dim3 grid((8 * lw + 1023) / 1024, nentries);
+    lwe_sum_xor_kernel<<<grid, 256, 0, s>>>(entries, lw);
     return cudaGetLastError();
 }
 

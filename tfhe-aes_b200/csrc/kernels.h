@@ -97,6 +97,16 @@ struct SumEntry {
     int _pad;
 };
 cudaError_t launch_lwe_sum(const SumEntry *entries, int nentries, int unit_words, cudaStream_t s);
+// gather-sum of a SumEntry plus a clear byte XORed into the encrypted destination byte (1-bit blocks): bit j of
+// (clear ^ *clear_src) adds bit << 63 to the body of LWE j
+struct SumXorEntry {
+    const uint64_t *src[5];
+    uint64_t *dst;
+    const uint8_t *clear_src;   // device byte, or nullptr
+    int nsrc;
+    uint32_t clear;
+};
+cudaError_t launch_lwe_sum_xor(const SumXorEntry *entries, int nentries, int lw, cudaStream_t s);
 cudaError_t launch_scale_lwe(const uint64_t *in, uint64_t *out, long nwords, uint64_t mul, cudaStream_t s);
 cudaError_t launch_sub_lwe(uint64_t *inout, const uint64_t *sub, long nwords, cudaStream_t s);
 cudaError_t launch_add_body(uint64_t *lwe, int lwe_words, int count, uint64_t add, cudaStream_t s);

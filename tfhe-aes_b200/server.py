@@ -67,3 +67,10 @@ class Server:
     def aes_ctr(self, encrypted_round_keys, encrypted_iv, number_of_outputs, first=0):
         """main.rs:55-64 — the CTR loop, all blocks in one batched call."""
         return self.engine.aes_ctr(encrypted_round_keys, encrypted_iv, first, number_of_outputs)
+
+    def aes_ctr_public_iv(self, encrypted_round_keys, iv, number_of_outputs, first=0, data=None):
+        """AES-CTR with the IV in the clear (only the AES key is encrypted): Enc(AES(iv + first + b) XOR data[b]) for
+        b < number_of_outputs; data None gives the bare keystream.  AES-128/192/256 follow from the number of round keys."""
+        rk = np.asarray(encrypted_round_keys)
+        rounds = rk.size // (16 * 8 * self.engine.lw) - 1
+        return self.engine.aes_ctr_public_iv([(rk, iv, first, number_of_outputs, data)], rounds)
