@@ -76,9 +76,10 @@ int tfa_ctx_synchronize(tfa_ctx *ctx);
  * 0 ks_decompose 1 ks_gemv 2 pbs 3 pfks_decompose 4 pfks_gemv 5 fourier 6 vp 7 cmux_tree 8 linear 9 misc */
 int tfa_ctx_profile(tfa_ctx *ctx, int enable);
 int tfa_ctx_profile_report(tfa_ctx *ctx, double *ms_per_stage /* [10] */, int *launch_groups /* [10] */);
-/* PBS kernel schedule (same arithmetic, SURVEY §9.4(3)): 0 = automatic (default), 1 = phase-synchronous kernel,
- * 2 = warp-specialised kernel, 3 = one ciphertext per two-CTA cluster (small batches), 4 = two ciphertext sets per CTA taking
- * turns (large batches; PARAM_OPT shape only).  For tests and measurements; unsupported shapes fall back to the automatic choice. */
+/* PBS kernel schedule (same arithmetic, SURVEY §9.4(3)): 0 = automatic (default), 2 = warp-specialised kernel, 3 = one
+ * ciphertext per two-CTA cluster (small batches), 4 = two ciphertext sets per CTA taking turns (large batches).  3 and 4 exist
+ * for glwe_dimension 4 only; at glwe_dimension 1 they run the warp-specialised kernel.  For tests and measurements.  Any other
+ * value returns TFA_ERR_PARAM and leaves the schedule unchanged. */
 int tfa_ctx_set_pbs_schedule(tfa_ctx *ctx, int schedule);
 /* DFMA microbenchmark: measured FP64 pipe peak of the device in TFLOP/s (roofline denominator) */
 int tfa_measure_fp64_peak(tfa_ctx *ctx, double *tflops);   /* max of the two below */

@@ -83,11 +83,12 @@ def test_bootstrap_matches_oracle(engine_test, oracle_test):
     assert np.array_equal(((ph + np.uint64(1 << 48)) >> np.uint64(49)) & np.uint64(1), msgs)
 
 
-@pytest.mark.parametrize("schedule", [1, 2])
+@pytest.mark.parametrize("schedule", [2])
 @pytest.mark.parametrize("count", [3, 9, 20])
 def test_bootstrap_both_kernel_schedules(engine_test, oracle_test, schedule, count):
-    """The phase-synchronous (1) and the warp-specialised (2) PBS kernels compute the same bootstrap; count 3 / 9 / 20
-    selects 1 / 4 / 8 ciphertexts per CTA at the test parameters."""
+    """The warp-specialised PBS kernel, forced with schedule 2, against the oracle; count 3 / 9 / 20 selects 1 / 4 / 8
+    ciphertexts per CTA at the test parameters.  Schedule 1, the phase-synchronous kernel, no longer exists: the same counts
+    run in test_bootstrap_after_rejected_pbs_schedules."""
     rng = np.random.default_rng(50 + count)
     o = oracle_test
     lut = rng.integers(0, 2 ** 64, 512, dtype=np.uint64)
@@ -98,6 +99,21 @@ def test_bootstrap_both_kernel_schedules(engine_test, oracle_test, schedule, cou
     finally:
         engine_test.set_pbs_schedule(0)
     assert torus_absdiff(o.phase_big(got), o.phase_big(o.bootstrap(lwe, lut))) < 2 ** 36
+
+
+@pytest.mark.parametrize("count", [3, 9, 20])
+def test_bootstrap_after_rejected_pbs_schedules(pkg, engine_test, oracle_test, count):
+    """Schedules other than 0, 2, 3 and 4 (1 included) are refused with TFA_ERR_PARAM and leave the automatic schedule in
+    place: the bootstrap that follows still matches the oracle with 1 / 4 / 8 ciphertexts per CTA."""
+    for schedule in (1, 5, -1):
+        with pytest.raises(pkg.TfaError) as ei:
+            engine_test.set_pbs_schedule(schedule)
+        assert ei.value.code == 1, schedule   # TFA_ERR_PARAM
+    rng = np.random.default_rng(50 + count)
+    o = oracle_test
+    lut = rng.integers(0, 2 ** 64, 512, dtype=np.uint64)
+    lwe = o.encrypt_lwe_small(rng.integers(0, 2 ** 64, count, dtype=np.uint64))
+    assert torus_absdiff(o.phase_big(engine_test.bootstrap(lwe, lut)), o.phase_big(o.bootstrap(lwe, lut))) < 2 ** 36
 
 
 def test_bootstrap_general_lut(engine_test, oracle_test):
@@ -387,28 +403,25 @@ def test_opt_bootstrap_matches_oracle(engine_opt, oracle_opt):
 
 
 @pytest.mark.parametrize("count", [150, 300])
-def test_opt_bootstrap_wave_both_schedules(engine_opt, oracle_opt, count):
-    """PARAM_OPT with 2 (count 150) and 3 (count 300) ciphertexts per CTA: both kernel schedules decrypt to the encrypted
-    bits, agree with each other on the phase, and a sample agrees with the oracle."""
+def test_opt_bootstrap_wave_ws_kernel(engine_opt, oracle_opt, count):
+    """PARAM_OPT with 2 (count 150) and 3 (count 300) ciphertexts per CTA of the warp-specialised kernel (forced schedule 2):
+    the outputs decrypt to the encrypted bits, and a sample agrees with the oracle."""
     o = oracle_opt
     rng = np.random.default_rng(count)
     msgs = rng.integers(0, 2, count).astype(np.uint64)
     ks = o.keyswitch(o.encrypt_bits(msgs))
     ks[:, -1] += np.uint64(1 << 62)
     lut = np.full(512, (1 << 64) - (1 << 48), dtype=np.uint64)
-    res = {}
-    for schedule in (1, 2):
-        engine_opt.set_pbs_schedule(schedule)
-        try:
-            res[schedule] = engine_opt.bootstrap(ks, lut)
-        finally:
-            engine_opt.set_pbs_schedule(0)
-        ph = o.phase_big(res[schedule]) + np.uint64(1 << 48)
-        assert np.array_equal(((ph + np.uint64(1 << 48)) >> np.uint64(49)) & np.uint64(1), msgs)
-    assert torus_absdiff(o.phase_big(res[1]), o.phase_big(res[2])) < 2 ** 36
+    engine_opt.set_pbs_schedule(2)
+    try:
+        got = engine_opt.bootstrap(ks, lut)
+    finally:
+        engine_opt.set_pbs_schedule(0)
+    ph = o.phase_big(got) + np.uint64(1 << 48)
+    assert np.array_equal(((ph + np.uint64(1 << 48)) >> np.uint64(49)) & np.uint64(1), msgs)
     sample = [0, count // 2, count - 1]
     ref = o.bootstrap(ks[sample], lut)
-    assert torus_absdiff(o.phase_big(res[2][sample]), o.phase_big(ref)) < 2 ** 36
+    assert torus_absdiff(o.phase_big(got[sample]), o.phase_big(ref)) < 2 ** 36
 
 
 @pytest.mark.parametrize("count,schedule", [(7, 4), (900, 0), (1400, 0)])

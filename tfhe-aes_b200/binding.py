@@ -262,8 +262,8 @@ class Engine:
     STAGES = ("ks_decompose", "ks_gemv", "pbs", "pfks_decompose", "pfks_gemv", "fourier", "vp", "cmux_tree", "linear", "misc")
 
     def set_pbs_schedule(self, schedule):
-        """0 = automatic, 1 = phase-synchronous PBS kernel, 2 = warp-specialised, 3 = one ciphertext per two-CTA cluster, 4 = two ciphertext
-        sets per CTA (include/tfhe_aes_b200.h: tfa_ctx_set_pbs_schedule)."""
+        """0 = automatic, 2 = warp-specialised PBS kernel, 3 = one ciphertext per two-CTA cluster, 4 = two ciphertext sets per CTA
+        (include/tfhe_aes_b200.h: tfa_ctx_set_pbs_schedule).  Any other value raises TfaError with code 1 (TFA_ERR_PARAM)."""
         self._ck(self.lib.tfa_ctx_set_pbs_schedule(self.h, int(schedule)))
 
     def profile(self, enable=True):

@@ -253,20 +253,6 @@ HD void phase_mac(int tid, CmuxSmem<K, G> &sm, CmuxRegs<K, G> &rg, const cd *__r
         }
     }
 }
-// one GGSW row (fixed level and row r) whose K+1 values for this thread's point are at w_ptr[c * 256]
-// (shared-memory ring slot filled by cp.async in the PBS kernel, or global memory in the emulation)
-template <int K, int G>
-HD void phase_mac_row(int tid, CmuxSmem<K, G> &sm, CmuxRegs<K, G> &rg, int r, const cd *w_ptr) {
-    cd w[K + 1];
-#pragma unroll
-    for (int c = 0; c <= K; c++) w[c] = w_ptr[c * POLY_M];
-#pragma unroll
-    for (int ct = 0; ct < G; ct++) {
-        const cd x = sm.xb[ct * (K + 1) + r][tid];
-#pragma unroll
-        for (int c = 0; c <= K; c++) cmac(rg.facc[ct][c], x, w[c]);
-    }
-}
 // software-pipelined form: operands of the NEXT row are fetched while the current row is computed
 template <int K, int G>
 struct MacOperands { cd w[K + 1]; cd x[G]; };

@@ -1,7 +1,6 @@
 // engine.cu — context, key preparation and the device-level stages of one WoPBS pass
 // (keyswitch -> PBS -> PFKS -> Fourier GGSW -> vertical packing), i.e. the GPU restatement of
 // many_wopbs_without_padding (many_wopbs.rs:31-116) batched over many encrypted bytes.
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include "engine.h"
@@ -123,8 +122,8 @@ extern "C" void tfa_ctx_destroy(tfa_ctx *ctx) {
 extern "C" const char *tfa_last_error(const tfa_ctx *ctx) { return ctx ? ctx->err.c_str() : g_create_error.c_str(); }
 extern "C" int tfa_ctx_synchronize(tfa_ctx *ctx) { CU(cudaStreamSynchronize(ctx->stream)); return TFA_OK; }
 extern "C" int tfa_ctx_set_pbs_schedule(tfa_ctx *ctx, int schedule) {
-    if (schedule < 0 || schedule > 4)
-        return ctx->fail(TFA_ERR_PARAM, "pbs schedule must be 0 (auto), 1 (phase-synchronous), 2 (warp-specialised), 3 (one PBS per two-CTA cluster) or 4 (two sets per CTA)");
+    if (schedule != 0 && (schedule < 2 || schedule > 4))
+        return ctx->fail(TFA_ERR_PARAM, "pbs schedule must be 0 (auto), 2 (warp-specialised), 3 (one PBS per two-CTA cluster) or 4 (two sets per CTA)");
     std::lock_guard<std::mutex> lk(ctx->mu);
     ctx->pbs_schedule = schedule;
     return TFA_OK;
@@ -301,27 +300,25 @@ int dev_pfks(tfa_ctx *ctx, const u64 *in, int count, u64 *out, int out_stride) {
     return TFA_OK;
 }
 
-// SURVEY §9.4(3)
+// SURVEY §9.4(3).  Three kernels of the same arithmetic (measured on B200, PARAM_OPT, 669 steps):
+//   pbs_ws2_kernel.cu  two sets of three ciphertexts per CTA taking turns: 18.9 ms per wave of 888 against 2 x 10.1 ms.  Whole
+//                      waves go to it, and so does a remainder of more than half a wave (pbs_ws_kernel would need two rounds of
+//                      148 CTAs for it: 20.2 ms).
+//   pbs_cl2_kernel.cu  one PBS per two-CTA cluster, levels transformed in parallel: at most one wave of clusters (74 ciphertexts)
+//                      -- key expansion stages, carry chain of few blocks, a single CTR block.
+//   pbs_ws_kernel.cu   warp-specialised, G ciphertexts per CTA (pick_G): a partial wave in 5-10 ms (10.6 ms per wave of 148 CTAs
+//                      at G = 3, 9.9 ms at G = 2, 7.5 ms at G = 1); every other batch, and every batch at K = 1.
+// Schedules 2, 3 and 4 force one of them (tfa_ctx_set_pbs_schedule); 3 and 4 exist at K = 4 only and fall back to pbs_ws_kernel.
 int dev_pbs(tfa_ctx *ctx, const u64 *in, int count, const u64 *lut, u64 in_scale, u64 pre_add, u64 post_add, u64 *out) {
     StageTimer t(ctx, ST_PBS);
     ctx->pbs_count += (u64)count;
     PbsArgs a{};
     a.lwe_in = in; a.bsk = ctx->bsk_f; a.tw = ctx->tw; a.lut = lut; a.out = out;
     a.in_scale = in_scale; a.pre_add_body = pre_add; a.post_add = post_add; a.lwe_dim = ctx->n; a.count = count;
-    // Two schedules of the same arithmetic (measured on B200, PARAM_OPT, 669 steps, one wave of 148 CTAs):
-    //   warp-specialised (pbs_ws_kernel.cu): 10.6 ms at G = 3, 9.9 ms at G = 2, 7.5 ms at G = 1
-    //   phase-synchronous (fp_kernels.cu):   13.1 ms at G = 3
-    // The warp-specialised kernel is the default wherever it is instantiated; the phase-synchronous one serves the
-    // remaining shapes (K = 1 test parameter sets with G > 1) and stays selectable for comparison.
-    static const bool timing = getenv("TFA_PBS_TIMING") != nullptr;
-    // Large batches: two sets of three ciphertexts per CTA taking turns (pbs_ws2_kernel.cu): 18.9 ms per wave of 888 against
-    // 2 x 10.1 ms.  Whole waves go to it, and so does a remainder of more than half a wave (the kernels below would need two rounds of
-    // 148 CTAs for it: 20.2 ms); a smaller remainder is served by the kernels below, which finish a partial wave in 5-10 ms.
-    static const bool no_ws2 = getenv("TFA_PBS_NO_WS2") != nullptr;
-    if (ctx->k == 4 && ctx->p.pbs_base_log == 8 && ctx->p.pbs_level == 5 && !timing &&
-        ((ctx->pbs_schedule == 0 && !no_ws2) || ctx->pbs_schedule == 4)) {
+    const int sched = ctx->pbs_schedule;
+    if (ctx->k == 4 && (sched == 0 || sched == 4)) {
         const int wave = 6 * ctx->sm_count;
-        int n2 = ctx->pbs_schedule == 4 ? count : (count / wave) * wave;
+        int n2 = sched == 4 ? count : (count / wave) * wave;
         if (count - n2 > wave / 2) n2 = count;
         if (n2 > 0) {
             PbsArgs b = a;
@@ -334,66 +331,8 @@ int dev_pbs(tfa_ctx *ctx, const u64 *in, int count, const u64 *lut, u64 in_scale
             a.count = count -= n2;
         }
     }
-    // Small batches (at most one wave of two-CTA clusters, 74 ciphertexts): one PBS per cluster, levels transformed in parallel
-    // (pbs_cl2_kernel.cu) -- key expansion stages, carry chain of few blocks, a single CTR block.
-    static const bool no_cluster = getenv("TFA_PBS_NO_CLUSTER") != nullptr;
-    if (ctx->k == 4 && ((ctx->pbs_schedule == 0 && count <= 74 && !no_cluster) || ctx->pbs_schedule == 3)) {
-        if (getenv("TFA_PBS_TIMING")) {   // debug aid: per-activity cycles of cluster 0 / CTA 0 (FFT thread 0, MAC thread 0)
-            uint64_t *d = nullptr, h[12];
-            CU(cudaMalloc(&d, sizeof(h)));
-            CU(cudaMemsetAsync(d, 0, sizeof(h), ctx->stream));
-            a.dbg = d;
-            CU(launch_pbs_cl2(a, ctx->stream));
-            CU(cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-            CU(cudaStreamSynchronize(ctx->stream));
-            cudaFree(d);
-            static const char *nm[12] = {"F:wait_acc", "F:decompose", "F:fwd_fft", "F:cluster_bar", "F:wait_inv", "F:inverse",
-                                         "M:wait_row", "M:row", "M:remote_store", "M:cluster_bar", "M:sum+handover", "-"};
-            fprintf(stderr, "[pbs_cl2 timing] cycles per CMux step:");
-            for (int k = 0; k < 11; k++) fprintf(stderr, " %s=%.0f", nm[k], (double)h[k] / ctx->n);
-            fprintf(stderr, "\n");
-            ctx->launches++;
-            return TFA_OK;
-        }
-        CU(launch_pbs_cl2(a, ctx->stream));
-        ctx->launches++;
-        return TFA_OK;
-    }
-    const int G = pick_G(ctx->k, count);
-    const bool ws_available = true;   // every (K, G) pick_G returns is instantiated in both kernels
-    const bool use_ws = ws_available && ctx->pbs_schedule != 1;
-    if (timing && G == 3 && ctx->k == 4) {
-        // debug aid: per-phase clock64() totals of block 0 (one thread per role)
-        uint64_t *d = nullptr;
-        static uint64_t h[16 + 3 * 512];
-        CU(cudaMalloc(&d, sizeof(h)));
-        CU(cudaMemsetAsync(d, 0, sizeof(h), ctx->stream));
-        a.dbg = d;
-        if (use_ws) CU(launch_pbs_ws(ctx->k, G, ctx->p.pbs_base_log, ctx->p.pbs_level, a, ctx->stream));
-        else CU(launch_pbs(ctx->k, G, ctx->p.pbs_base_log, ctx->p.pbs_level, a, ctx->stream));
-        CU(cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(d);
-        static const char *nm[9] = {"decompose", "fwd_fft", "bar_after_fwd", "wait_full", "mac", "bar_after_mac", "inv0+bar", "inv_fft", "bar_end"};
-        static const char *nw[9] = {"F:decompose", "F:digits+pass1", "F:wait_empty", "F:store+pass2+store", "F:wait_inv", "F:inverse",
-                                    "M:wait", "M:mac", "M:handover"};
-        fprintf(stderr, "[pbs timing] cycles per CMux step (block 0):");
-        for (int k = 0; k < 9; k++) fprintf(stderr, " %s=%.0f", use_ws ? nw[k] : nm[k], (double)h[k] / ctx->n);
-        fprintf(stderr, "\n");
-        if (use_ws && getenv("TFA_PBS_TRACE")) {   // event times of steps 100..103: FFT group 0, FFT group 14, MAC thread 0
-            uint64_t t0 = ~0ull;
-            for (int k = 16; k < 16 + 3 * 512; k++) if (h[k] && h[k] < t0) t0 = h[k];
-            for (int sec = 0; sec < 3; sec++) {
-                fprintf(stderr, "[pbs trace] %s:", sec == 0 ? "fft_g0" : sec == 1 ? "fft_g14" : "mac");
-                for (int k = 0; k < 512 && h[16 + sec * 512 + k]; k++) fprintf(stderr, " %llu", (unsigned long long)(h[16 + sec * 512 + k] - t0));
-                fprintf(stderr, "\n");
-            }
-        }
-        ctx->launches++;
-        return TFA_OK;
-    }
-    if (use_ws) CU(launch_pbs_ws(ctx->k, G, ctx->p.pbs_base_log, ctx->p.pbs_level, a, ctx->stream));
-    else CU(launch_pbs(ctx->k, G, ctx->p.pbs_base_log, ctx->p.pbs_level, a, ctx->stream));
+    if (ctx->k == 4 && ((sched == 0 && count <= 74) || sched == 3)) CU(launch_pbs_cl2(a, ctx->stream));
+    else CU(launch_pbs_ws(ctx->k, pick_G(ctx->k, count), ctx->p.pbs_base_log, ctx->p.pbs_level, a, ctx->stream));
     ctx->launches++;
     return TFA_OK;
 }

@@ -43,7 +43,7 @@ struct tfa_ctx {
 
     // optional per-stage GPU timing (tfa_ctx_profile): events around every launch group
     bool profiling;
-    int pbs_schedule;      // 0 auto, 1 phase-synchronous, 2 warp-specialised, 3 cluster pair per ciphertext, 4 two sets per CTA (tfa_ctx_set_pbs_schedule)
+    int pbs_schedule;      // 0 auto, 2 warp-specialised, 3 cluster pair per ciphertext, 4 two sets per CTA (tfa_ctx_set_pbs_schedule)
     struct ProfRec { int stage; cudaEvent_t a, b; };
     std::vector<ProfRec> prof;
 

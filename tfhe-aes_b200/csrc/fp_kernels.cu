@@ -1,6 +1,5 @@
-// fp_kernels.cu — the FP64 kernels of the WoPBS chain (sm_100a):
-//   pbs_kernel            blind rotation + sample extract (PBS) — K3 of SURVEY.md §2.2
-//                         (circuit_bootstrap_boolean -> bootstrap, many_wopbs.rs:253; extract_bits loop :194)
+// fp_kernels.cu — the FP64 kernels of the WoPBS chain other than the PBS (sm_100a).  The PBS, K3 of SURVEY.md §2.2,
+// has kernels of its own: pbs_ws_kernel.cu, pbs_ws2_kernel.cu and pbs_cl2_kernel.cu.
 //   vp_kernel             blind-rotation half of vertical_packing + sample extract — K6 (many_wopbs.rs:277)
 //   cmux_tree_kernel      one layer of the vertical-packing CMux tree (LUT larger than N) — K6 general form
 //   fourier_convert_kernel standard GGSW -> Fourier layout — K5 (fill_with_forward_fourier, many_wopbs.rs:263)
@@ -54,183 +53,6 @@ __device__ __forceinline__ void sample_extract(int tid, const CmuxSmem<K, G> &sm
         out[idx] = (j == 0) ? sm.acc[g][r][0] : (uint64_t)0 - sm.acc[g][r][POLY_N - j];
     }
     if (tid == 0) out[K * POLY_N] = sm.acc[g][K][0] + post_add;
-}
-
-// ------------------------------------------------------------------------------------------------
-// PBS: out[ct] = SampleExtract( BlindRotate(lut * X^-b~, a~, BSK) ) + post_add on the body
-//
-// Bootstrap-key streaming: the Fourier BSK slice of one CMux step is LEVELS x (K+1) rows of (K+1) x 4 KB
-// (K=4: 25 rows x 20 KB), stored in consumption order, each row [col][p] contiguous.  Rows are streamed
-// L2 -> shared memory by the TMA engine (cp.async.bulk, one copy per row issued by ONE lane) into a ring that
-// holds exactly one level (K+1 slots).  One FULL mbarrier counts the K+1 rows of a level (arrive.expect_tx per
-// row + transaction bytes); every thread waits on it ONCE per level, before the multiply-accumulate phase, and
-// then runs the K+1 rows back to back.  Slots are handed back row by row: each warp arrives on the slot's
-// EMPTY mbarrier after its multiply-accumulate of the row, and one lane (the role rotates over the warps)
-// refills the slot freed one row earlier with the same row of the next level; the last slot of a level is
-// refilled right after the CTA barrier that ends the phase.  So the key for level l+1 is requested while level
-// l is being consumed and lands during the FFT phase in between; no thread spends issue slots or LSU
-// wavefronts on the copy (the per-thread cp.async ring of the first build cost 8 % of all instructions and
-// 37 % of the shared-memory wavefronts of the kernel, profiles/r1_pbs_source_phases.txt).  All CTAs walk the
-// key in the same order, so HBM sees the key once per wave and L2 serves the other CTAs.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t *bar, unsigned bytes) {
-    asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n\t}" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, unsigned parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra.uni WAIT_DONE;\n\t"
-        "bra.uni WAIT_LOOP;\n\t"
-        "WAIT_DONE:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-// one bulk copy global -> shared (TMA engine), completion counted in bytes on `bar`
-__device__ __forceinline__ void bulk_copy_g2s(void *smem_dst, const void *gmem_src, unsigned bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
-                 "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-
-template <int K, int G>
-struct PbsSmemLayout {
-    static constexpr size_t ROW_ELEMS = (size_t)POLY_M * (K + 1);
-    static constexpr size_t ring_off = (sizeof(CmuxSmem<K, G>) + 127) & ~(size_t)127;
-    static constexpr size_t bar_off = ring_off + (K + 1) * ROW_ELEMS * sizeof(cd);   // FULL, EMPTY[K+1]
-    static constexpr size_t bytes = bar_off + (K + 2) * sizeof(uint64_t);
-};
-
-// modulus switch to 2N (SURVEY §9.4(3)): a~ = (a * in_scale [+ pre_add on the body] + 2^53) >> 54
-__device__ __forceinline__ int mod_switch_2n(const PbsArgs &a, int ct, int i) {
-    uint64_t x = a.lwe_in[(size_t)ct * (a.lwe_dim + 1) + i] * a.in_scale;
-    if (i == a.lwe_dim) x += a.pre_add_body;
-    return (int)((x + (1ull << 53)) >> 54) & (2 * POLY_N - 1);
-}
-
-// TIMING = true (debug builds of the launcher only, PbsArgs::dbg != nullptr): thread 0 accumulates clock64() deltas per
-// phase in shared memory and block 0 writes them to dbg[0..PT_COUNT).
-enum { PT_DECOMP, PT_FWD, PT_BAR_FWD, PT_WAIT_FULL, PT_MAC, PT_BAR_MAC, PT_INV0, PT_INV, PT_BAR_END, PT_COUNT };
-template <int K, int G, int BASE_LOG, int LEVELS, bool TIMING = false>
-__global__ void __launch_bounds__(CMUX_THREADS, 1) pbs_kernel(PbsArgs a) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ long long tacc[PT_COUNT];
-    long long tlast = 0;
-#define PT(k) do { if (TIMING && threadIdx.x == 0) { const long long t_ = clock64(); tacc[k] += t_ - tlast; tlast = t_; } } while (0)
-    typedef PbsSmemLayout<K, G> L;
-    CmuxSmem<K, G> &sm = smem_view<K, G>(smem_raw);
-    constexpr int RING = K + 1;                          // one level of the GGSW
-    constexpr int ROWS = LEVELS * (K + 1);               // GGSW rows per CMux step, stored in consumption order
-    constexpr int ROW_ELEMS = (int)L::ROW_ELEMS;
-    constexpr unsigned ROW_BYTES = (unsigned)(ROW_ELEMS * sizeof(cd));
-    cd *ring = reinterpret_cast<cd *>(smem_raw + L::ring_off);                 // [RING][K+1][256]
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw + L::bar_off);      // one per level
-    uint64_t *empty = full + 1;                                                // [RING]
-    CmuxRegs<K, G> rg;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int n = a.lwe_dim;
-    const int ct0 = blockIdx.x * G;
-    const int nrows = n * ROWS;
-    // fetch row q into slot q % RING (the caller knows the slot is free)
-    auto produce = [&](int q) {
-        const int slot = q % RING;
-        mbar_arrive_expect_tx(full, ROW_BYTES);
-        bulk_copy_g2s(ring + (size_t)slot * ROW_ELEMS, a.bsk + (size_t)q * ROW_ELEMS, ROW_BYTES, full);
-    };
-    if (tid == 0) {
-        mbar_init(full, RING);
-        for (int s = 0; s < RING; s++) mbar_init(&empty[s], CMUX_THREADS / 32);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (tid == 0)
-        for (int q = 0; q < RING; q++) produce(q);       // nrows >= RING always (n >= 1, LEVELS >= 1)
-
-    load_twiddles<K, G>(sm, a.tw, tid);
-    for (int g = 0; g < G; g++) {
-        const int bhat = mod_switch_2n(a, min(ct0 + g, a.count - 1), n);
-        const int rot = (2 * POLY_N - bhat) & (2 * POLY_N - 1);
-        for (int idx = tid; idx < (K + 1) * POLY_N; idx += CMUX_THREADS) {
-            const int r = idx / POLY_N, j = idx % POLY_N;
-            sm.acc[g][r][j] = (r == K) ? rotated_coef(a.lut, j, rot) : 0;
-        }
-    }
-    // thread g < G tracks the rotation of ciphertext g: the mask element of the NEXT step is loaded from global
-    // memory one step ahead, so its latency hides behind a whole CMux
-    const int my_ct = min(ct0 + min(tid, G - 1), a.count - 1);
-    int next_rot = 0;
-    if (tid < G) sm.rot[tid] = mod_switch_2n(a, my_ct, 0);
-    if (TIMING && tid == 0) { for (int k = 0; k < PT_COUNT; k++) tacc[k] = 0; tlast = clock64(); }
-    __syncthreads();
-    int q = 0;                                           // next row to consume (uniform over the CTA)
-    unsigned level_parity = 0;
-#pragma unroll 1
-    for (int i = 0; i < n; i++) {
-        // a step whose rotations are all zero adds exactly zero (ct1 == 0): it is executed like any
-        // other so that the key walk stays in lock-step with the ring
-        if (tid < G && i + 1 < n) next_rot = mod_switch_2n(a, my_ct, i + 1);
-        phase_load_decompose<K, G, BASE_LOG, LEVELS, DIFF_ROTATE>(tid, sm, rg, nullptr);
-        PT(PT_DECOMP);
-#pragma unroll 1
-        for (int lev = LEVELS; lev >= 1; lev--) {
-            phase_fwd1<K, G>(tid, sm, rg);
-            __syncwarp();
-            phase_fwd2<K, G>(tid, sm, rg);
-            __syncwarp();
-            phase_fwd3<K, G>(tid, sm, rg);
-            PT(PT_FWD);
-            __syncthreads();
-            PT(PT_BAR_FWD);
-            mbar_wait(full, level_parity);               // the K+1 rows of this level have landed
-            level_parity ^= 1;
-            PT(PT_WAIT_FULL);
-#pragma unroll
-            for (int r = 0; r <= K; r++, q++) {
-                phase_mac_row<K, G>(tid, sm, rg, r, ring + (size_t)r * ROW_ELEMS + tid);
-                __syncwarp();
-                if (lane == 0) {
-                    // the warp's reads of slot r are complete (their values fed the FMAs above)
-                    if (r < K) mbar_arrive(&empty[r]);
-                    // refill the slot freed one row earlier, once every warp has released it
-                    if (r >= 1 && warp == (q & (CMUX_THREADS / 32 - 1)) && q - 1 + RING < nrows) {
-                        mbar_wait(&empty[r - 1], (level_parity ^ 1) & 1);
-                        produce(q - 1 + RING);
-                    }
-                }
-                // the digits of the next level (integer + conversion pipes) are extracted in the shadow of the
-                // multiply-accumulate (FP64 pipe): v is free during this phase
-                if (r == 0 && lev > 1) phase_next_digits<K, G, BASE_LOG, LEVELS>(tid, rg, lev - 1);
-            }
-            PT(PT_MAC);
-            __syncthreads();
-            // every warp is past the phase: the last slot is free
-            if (tid == 0 && q - 1 + RING < nrows) produce(q - 1 + RING);
-            PT(PT_BAR_MAC);
-        }
-        phase_inv0<K, G>(tid, sm, rg);
-        __syncthreads();
-        PT(PT_INV0);
-        phase_inv1<K, G>(tid, sm, rg);
-        __syncwarp();
-        phase_inv2<K, G>(tid, sm, rg);
-        __syncwarp();
-        phase_inv3<K, G>(tid, sm, rg);
-        if (tid < G) sm.rot[tid] = next_rot;
-        PT(PT_INV);
-        __syncthreads();
-        PT(PT_BAR_END);
-    }
-    if (TIMING && tid == 0 && blockIdx.x == 0)
-        for (int k = 0; k < PT_COUNT; k++) a.dbg[k] = (uint64_t)tacc[k];
-#undef PT
-    for (int g = 0; g < G; g++)
-        if (ct0 + g < a.count) sample_extract<K, G>(tid, sm, g, a.out + (size_t)(ct0 + g) * (K * POLY_N + 1), a.post_add);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -342,26 +164,6 @@ static cudaError_t set_smem(F f, size_t bytes) {
     return cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
-#define LAUNCH_PBS(k, g, bl, lv)                                                               \
-    if (K == k && G == g && base_log == bl && levels == lv) {                                  \
-        const size_t smem = PbsSmemLayout<k, g>::bytes;                                        \
-        cudaError_t e = set_smem(pbs_kernel<k, g, bl, lv>, smem);                              \
-        if (e != cudaSuccess) return e;                                                        \
-        pbs_kernel<k, g, bl, lv><<<(a.count + g - 1) / g, CMUX_THREADS, smem, s>>>(a);         \
-        return cudaGetLastError();                                                             \
-    }
-cudaError_t launch_pbs(int K, int G, int base_log, int levels, const PbsArgs &a, cudaStream_t s) {
-    if (a.dbg && K == 4 && G == 3 && base_log == 8 && levels == 5) {   // per-phase cycle counts (TFA_PBS_TIMING=1)
-        const size_t smem = PbsSmemLayout<4, 3>::bytes;
-        cudaError_t e = set_smem(pbs_kernel<4, 3, 8, 5, true>, smem);
-        if (e != cudaSuccess) return e;
-        pbs_kernel<4, 3, 8, 5, true><<<(a.count + 2) / 3, CMUX_THREADS, smem, s>>>(a);
-        return cudaGetLastError();
-    }
-    LAUNCH_PBS(4, 1, 8, 5) LAUNCH_PBS(4, 2, 8, 5) LAUNCH_PBS(4, 3, 8, 5)
-    LAUNCH_PBS(1, 1, 8, 5) LAUNCH_PBS(1, 4, 8, 5) LAUNCH_PBS(1, 8, 8, 5)
-    return cudaErrorInvalidValue;
-}
 #define LAUNCH_VP(k, g, bl, lv)                                                      \
     if (K == k && G == g && base_log == bl && levels == lv) {                        \
         size_t smem = sizeof(CmuxSmem<k, g>);                                        \

@@ -14,7 +14,7 @@ struct PbsArgs {
     uint64_t post_add;        // added to the output body
     int lwe_dim;
     int count;
-    uint64_t *dbg;            // debug: per-phase cycle counters of block 0 (nullptr in production)
+    uint64_t *dbg;            // per-activity cycle counters of CTA 0 in the WS_TIMING / WS2_TIMING builds of scratch/pbs_lab (nullptr otherwise)
 };
 struct VpArgs {
     const double2 *ggsw_f;    // [njobs][nbits][level][row][col][p], bit 0 = LSB
@@ -77,7 +77,6 @@ bool tc5_ks_supported(int ncols, int key_pitch_cols, int rows_pad);
 cudaError_t launch_tc5_keyswitch(const int8_t *dl, int rows_pad, const uint64_t *key, int rows, int ncols, int key_pitch_cols, int count,
                                  const uint64_t *in, int in_stride, int body_index, uint64_t *out, int out_stride, cudaStream_t s);
 
-cudaError_t launch_pbs(int K, int G, int base_log, int levels, const PbsArgs &a, cudaStream_t s);
 cudaError_t launch_pbs_ws(int K, int G, int base_log, int levels, const PbsArgs &a, cudaStream_t s);
 cudaError_t launch_pbs_ws2(int K, int G, int base_log, int levels, const PbsArgs &a, cudaStream_t s);   // K = 4, G = 3, (2^8, 5): two sets of G per CTA (large batches)
 cudaError_t launch_pbs_cl2(const PbsArgs &a, cudaStream_t s);   // K = 4, (2^8, 5): one ciphertext per cluster of two CTAs (small batches)

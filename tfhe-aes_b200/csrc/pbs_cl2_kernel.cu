@@ -81,7 +81,7 @@ __device__ __forceinline__ double digit_of_level(uint64_t x, int lev) {
 }
 
 // NP = own polynomials of this CTA (3 for rank 0, 2 for rank 1)
-template <int NP, bool TIMING>
+template <int NP>
 __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const unsigned rank) {
     const int tid = threadIdx.x;
     const unsigned peer = rank ^ 1u;
@@ -91,10 +91,6 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
     const int ct = blockIdx.x >> 1;
     const int n = a.lwe_dim;
     constexpr int ROW_ELEMS = (CL_K + 1) * POLY_M;
-    // debug timing (a.dbg != nullptr): clock64() deltas per activity of FFT thread 0 / MAC thread 0 of CTA 0, written to dbg[0..12)
-    const bool timing = TIMING && blockIdx.x == 0 && (tid == 0 || tid == 256);
-    long long tacc[6] = {0, 0, 0, 0, 0, 0}, tlast = timing ? clock64() : 0;
-#define CT(k) do { if (TIMING && timing) { const long long t_ = clock64(); tacc[k] += t_ - tlast; tlast = t_; } } while (0)
 
     if (tid < 256) {
         // ================================ FFT groups ========================================================================
@@ -116,7 +112,6 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
                 const uint64_t raw_next = a.lwe_in[(size_t)ct * (n + 1) + min(i + 1, n - 1)];
                 if (i > 0) ws_mbar_wait_lane(&sm.accready[lp], (unsigned)(i - 1) & 1);   // lanes of one warp may belong to two polynomials
                 __syncwarp();
-                CT(0);
                 // rotated difference acc * X^rot - acc, digit of this group's level only (load_decompose_rot of cmux_core.cuh)
                 const int s0 = (lane - rot) & (2 * POLY_N - 1);
 #pragma unroll
@@ -131,7 +126,6 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
                     const uint64_t a1 = ((x1 ^ m1) - m1) - poly[j + POLY_M];
                     v[n1] = cmk(digit_of_level(a0, lev), digit_of_level(a1, lev));
                 }
-                CT(1);
                 fft256_fwd_pass1_compute(v, lane, sm.tw);
                 if (active) fft256_fwd_pass1_store(v, lane, slot);
                 __syncwarp();
@@ -143,11 +137,9 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
                 }
                 __syncwarp();
                 if (active && lane == 0) ws_mbar_arrive(&sm.allspec);
-                CT(2);
                 rot = (int)((raw_next * a.in_scale + (1ull << 53)) >> 54) & (2 * POLY_N - 1);
                 if (warp_owner) {
                     ws_mbar_wait(&sm.inv, (unsigned)i & 1);
-                    CT(4);
 #pragma unroll
                     for (int k2 = 0; k2 < 16; k2++) v[k2] = slot[lane + 16 * k2];
                     fft256_inv_pass1_compute(v);
@@ -165,11 +157,9 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
                     }
                     __syncwarp();
                     if (owner && lane == 0) ws_mbar_arrive(&sm.accready[lp]);
-                    CT(5);
                 }
             }
         }
-        if (timing) for (int k = 0; k < 6; k++) a.dbg[k] = (uint64_t)tacc[k];
     } else {
         // ================================ MAC role ==========================================================================
         // One ciphertext per cluster: every key value is used exactly once per CTA, so the key rows are not staged in shared
@@ -197,7 +187,6 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
 #pragma unroll
             for (int c = 0; c <= CL_K; c++) facc[c] = cmk(0.0, 0.0);
             ws_mbar_wait(&sm.allspec, (unsigned)i & 1);
-            CT(0);
             const int inext = min(i + 1, n - 1);          // the last step prefetches rows it never uses
 #pragma unroll
             for (int g = 0; g < NROWS; g++) {
@@ -220,16 +209,13 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
 #pragma unroll
                     for (int c = 0; c <= CL_K; c++) wbuf[r][c] = t[r][c];
             }
-            CT(1);
             // partial sums of the peer's columns -> its shared memory; the bytes complete its rxfull barrier as they land
 #pragma unroll
             for (int c = 0; c < PEER_NP; c++)
                 st_async_cd(remote_rx + (unsigned)(((i & 1) * CL_MAXP + c) * POLY_M * sizeof(cd)), facc[peer_pbase + c], remote_bar);
-            CT(2);
             mbar_wait_cluster(&sm.rxfull, (unsigned)i & 1);
             // the next phase expects the peer's NP columns again (posted thousands of cycles before the peer can send them)
             if (p == 0) ws_mbar_arrive_expect_tx(&sm.rxfull, (unsigned)(NP * POLY_M * sizeof(cd)));
-            CT(3);
 #pragma unroll
             for (int c = 0; c < NP; c++) {
                 const cd r = sm.rx[i & 1][c][p];
@@ -237,14 +223,10 @@ __device__ __forceinline__ void cl2_body(const PbsArgs &a, ClSmem &sm, const uns
             }
             __syncwarp();
             if (mlane == 0) ws_mbar_arrive(&sm.inv);
-            CT(4);
         }
-        if (timing) for (int k = 0; k < 6; k++) a.dbg[6 + k] = (uint64_t)tacc[k];
     }
-#undef CT
 }
 
-template <bool TIMING>
 __global__ void __launch_bounds__(CL_THREADS, 1) pbs_cl2_kernel(PbsArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     ClSmem &sm = *reinterpret_cast<ClSmem *>(smem_raw);
@@ -272,8 +254,8 @@ __global__ void __launch_bounds__(CL_THREADS, 1) pbs_cl2_kernel(PbsArgs a) {
     }
     __syncthreads();
     cluster_sync_all();                               // both CTAs are resident and their barriers initialised before any remote access
-    if (rank == 0) cl2_body<3, TIMING>(a, sm, rank);
-    else cl2_body<2, TIMING>(a, sm, rank);
+    if (rank == 0) cl2_body<3>(a, sm, rank);
+    else cl2_body<2>(a, sm, rank);
     __syncthreads();
     cluster_sync_all();                               // no CTA leaves while its peer may still write into its shared memory
     // sample extract of coefficient 0 (SURVEY §9.4(3)): mask segment r from polynomial r, body from polynomial K
@@ -290,8 +272,7 @@ __global__ void __launch_bounds__(CL_THREADS, 1) pbs_cl2_kernel(PbsArgs a) {
 // one cluster of two CTAs per ciphertext: worthwhile for count <= 74 (one wave)
 cudaError_t launch_pbs_cl2(const PbsArgs &a, cudaStream_t s) {
     const size_t smem = sizeof(ClSmem);
-    auto kernel = a.dbg ? pbs_cl2_kernel<true> : pbs_cl2_kernel<false>;   // a.dbg: per-activity cycle counters (TFA_PBS_TIMING)
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(pbs_cl2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2 * a.count);
@@ -303,5 +284,5 @@ cudaError_t launch_pbs_cl2(const PbsArgs &a, cudaStream_t s) {
     attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, a);
+    return cudaLaunchKernelEx(&cfg, pbs_cl2_kernel, a);
 }

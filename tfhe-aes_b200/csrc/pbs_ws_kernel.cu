@@ -1,6 +1,6 @@
 // pbs_ws_kernel.cu — warp-specialised PBS (blind rotation + sample extract), sm_100a.
 //
-// Same arithmetic as pbs_kernel (fp_kernels.cu / cmux_core.cuh), different schedule.  One CTA of 512
+// The CMux arithmetic of cmux_core.cuh, in a warp-specialised schedule.  One CTA of 512
 // threads holds G ciphertexts for all n CMux steps:
 //   warps 8-15 "FFT warps" : per step: rotate-subtract + signed decomposition, per level a forward FFT of
 //                            every digit polynomial into its hand-over slot, then the K+1 inverse FFTs and the
@@ -54,6 +54,9 @@
 #ifndef WS_DIAG
 #define WS_DIAG 0         // diagnostics of scratch/pbs_lab: each bit removes one piece of work (results are WRONG when != 0)
 #endif
+#ifndef WS_TIMING
+#define WS_TIMING 0       // scratch/pbs_lab: per-activity clock64() sums of CTA 0 (FFT thread 0, MAC thread 0) into PbsArgs::dbg[0..WT_COUNT)
+#endif
 namespace PBS_WS_NS {
 
 template <int K, int G>
@@ -86,18 +89,13 @@ __device__ __forceinline__ void cmac_cols(cd (&facc)[G][KP1], int c, const cd (&
     for (int g = 0; g < G; g++) facc[g][c].y = fma(x[g].y, w.x, facc[g][c].y);
 }
 
-// TIMING (debug launches, PbsArgs::dbg != nullptr): thread 0 (FFT role) and thread 256 (MAC role) of block 0 accumulate
-// clock64() deltas per activity and write them to dbg[0..WT_COUNT).
 enum { WT_F_DECOMP, WT_F_PASS1, WT_F_WAIT_EMPTY, WT_F_POST, WT_F_WAIT_INV, WT_F_INV, WT_M_WAIT, WT_M_MAC, WT_M_HANDOVER, WT_COUNT };
-template <int K, int G, int BASE_LOG, int LEVELS, bool TIMING = false>
+template <int K, int G, int BASE_LOG, int LEVELS>
 __global__ void __launch_bounds__(WS_THREADS, 1) pbs_ws_kernel(PbsArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     long long tacc[6] = {0, 0, 0, 0, 0, 0};
-    long long tlast = TIMING ? clock64() : 0;
-#define WT(k) do { if (TIMING) { const long long t_ = clock64(); tacc[(k) % 6] += t_ - tlast; tlast = t_; \
-                              if (trace_on && trace_idx < 512) a.dbg[16 + trace_sec * 512 + trace_idx++] = (uint64_t)t_; } } while (0)
-    int trace_sec = 0, trace_idx = 0;
-    bool trace_on = false;
+    long long tlast = WS_TIMING ? clock64() : 0;
+#define WT(k) do { if (WS_TIMING) { const long long t_ = clock64(); tacc[(k) % 6] += t_ - tlast; tlast = t_; } } while (0)
     WsSmem<K, G> &sm = *reinterpret_cast<WsSmem<K, G> *>(smem_raw);
     const int tid = threadIdx.x;
     const int n = a.lwe_dim;
@@ -197,7 +195,6 @@ __global__ void __launch_bounds__(WS_THREADS, 1) pbs_ws_kernel(PbsArgs a) {
 #if !WS_ROT_LATE
                 const int rot_next = (i + 1 < n) ? ws_mod_switch_2n(a, my_ct, i + 1) : 0;
 #endif
-                if (TIMING) { trace_on = blockIdx.x == 0 && (ftid == 0 || ftid == 224) && i >= 100 && i < 104; trace_sec = ftid == 0 ? 0 : 1; }
                 load_decompose_rot<BASE_LOG, LEVELS>(sm.acc[ct][r], lane, rot, v, st_re, st_im);
 #if WS_TMEM_ST
                 // park the digits of levels 4..1: per level one word per four coefficients (8 words), 32 columns per thread
@@ -300,7 +297,7 @@ __global__ void __launch_bounds__(WS_THREADS, 1) pbs_ws_kernel(PbsArgs a) {
 #endif
                 WT(WT_F_INV);
             }
-            if (TIMING && blockIdx.x == 0 && ftid == 0)
+            if (WS_TIMING && a.dbg && blockIdx.x == 0 && ftid == 0)
                 for (int k = 0; k < 6; k++) a.dbg[k] = (uint64_t)tacc[k];
         }
     } else {
@@ -328,7 +325,6 @@ __global__ void __launch_bounds__(WS_THREADS, 1) pbs_ws_kernel(PbsArgs a) {
         int q = 0;                                // next key row to consume
 #pragma unroll 1
         for (int i = 0; i < n_mac; i++) {
-            if (TIMING) { trace_on = blockIdx.x == 0 && p == 0 && i >= 100 && i < 104; trace_sec = 2; }
 #pragma unroll
             for (int g = 0; g < G; g++)
 #pragma unroll
@@ -413,7 +409,7 @@ __global__ void __launch_bounds__(WS_THREADS, 1) pbs_ws_kernel(PbsArgs a) {
             }
             WT(WT_M_HANDOVER);
         }
-        if (TIMING && blockIdx.x == 0 && p == 0)
+        if (WS_TIMING && a.dbg && blockIdx.x == 0 && p == 0)
             for (int k = 6; k < WT_COUNT; k++) a.dbg[k] = (uint64_t)tacc[k % 6];
     }
 #undef WT
@@ -449,13 +445,6 @@ using namespace PBS_WS_NS;
         return cudaGetLastError();                                                                      \
     }
 cudaError_t PBS_WS_LAUNCH_NAME(int K, int G, int base_log, int levels, const PbsArgs &a, cudaStream_t s) {
-    if (a.dbg && K == 4 && G == 3 && base_log == 8 && levels == 5) {   // per-activity cycle counts (TFA_PBS_TIMING=1)
-        const size_t smem = sizeof(WsSmem<4, 3>);
-        cudaError_t e = cudaFuncSetAttribute(pbs_ws_kernel<4, 3, 8, 5, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        pbs_ws_kernel<4, 3, 8, 5, true><<<(a.count + 2) / 3, WS_THREADS, smem, s>>>(a);
-        return cudaGetLastError();
-    }
     LAUNCH_WS(4, 1, 8, 5) LAUNCH_WS(4, 2, 8, 5) LAUNCH_WS(4, 3, 8, 5)
     LAUNCH_WS(1, 1, 8, 5) LAUNCH_WS(1, 4, 8, 5) LAUNCH_WS(1, 8, 8, 5)
     return cudaErrorInvalidValue;
