@@ -151,6 +151,27 @@ typedef struct tfa_ctr_stream {
 int tfa_aes_ctr_public_iv(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, uint64_t *out);
 /* streams: host array whose round_keys and data are device pointers; out: device; asynchronous on the context stream */
 int tfa_aes_ctr_public_iv_dev(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, uint64_t *out);
+/* AES-CTR with ENCRYPTED initial counter blocks (the CTR loop of main.rs:55-64) for nstreams independent streams in one call, each with
+ * its own AES key, encrypted IV and counter range; the streams share the context's FHE keys.  Output block b of stream s =
+ * Enc( AES_K_s(IV_s + first_s + b mod 2^128) XOR data_s[b] ), in stream order: out [sum of nblk][16][8][lw].  rounds = 10 / 12 / 14
+ * (AES-128 / 192 / 256), shared by all streams; round_keys of each stream [rounds + 1][16][8][lw]; iv_ct [16][8][lw]; data NULL: the
+ * bare keystream.  Streams whose iv_ct is the same pointer share one IV: its 128 bits are circuit-bootstrapped once.  Every stage of
+ * the counter add and every round runs over all blocks of the call at once: 128 * (distinct iv_ct) + (128 * rounds + 15) * (sum of
+ * nblk) PBS, which for one stream equals tfa_aes_ctr.
+ * Errors: TFA_ERR_PARAM for nstreams < 1, an nblk < 1, a NULL round_keys or iv_ct, a NULL out, more than INT_MAX / 16 blocks in all
+ * or another rounds; TFA_ERR_STATE without keys; TFA_ERR_UNSUPPORTED unless blocks carry one bit.  The context stays usable. */
+typedef struct tfa_ctr_enc_stream {
+    const uint64_t *round_keys;   /* [rounds + 1][16][8][lw] */
+    const uint64_t *iv_ct;        /* [16][8][lw] encrypted initial counter block */
+    const uint8_t *data;          /* [nblk][16] clear bytes XORed into the output, or NULL */
+    uint64_t first_lo, first_hi;  /* block b encrypts iv + first + b (mod 2^128) */
+    int32_t nblk;
+    int32_t _pad;
+} tfa_ctr_enc_stream;             /* 48 bytes, no implicit padding */
+/* host pointers; every distinct round-key and iv_ct buffer is copied once; synchronises before returning */
+int tfa_aes_ctr_streams(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, int nstreams, int rounds, uint64_t *out);
+/* streams: host array whose round_keys, iv_ct and data are device pointers; out: device; asynchronous on the context stream */
+int tfa_aes_ctr_streams_dev(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, int nstreams, int rounds, uint64_t *out);
 /* one AES round on nblk states (BASELINE config 2): 16*nblk many_sbox + ShiftRows/MixColumns + AddRoundKey */
 int tfa_aes_round(tfa_ctx *ctx, const uint64_t *round_key, uint64_t *states, int nblk);
 /* linear layers alone (server.rs:278-282, mix_columns.rs:4, inv_mix_columns.rs:4, shift_rows.rs:5, inv_shift_rows.rs:5) */

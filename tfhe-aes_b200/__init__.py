@@ -7,7 +7,7 @@ through `load_package()` in the repo-root `__graft_entry__.py`, or put this dire
 reference interface used by tests and bench.py.
 """
 from .binding import (  # noqa: F401
-    Engine, Params, TfaCtrStream, TfaError, param_opt, param_test, param_test2, gen_lut, lut_size, lib_path, load_library,
+    Engine, Params, TfaCtrStream, TfaCtrEncStream, TfaError, param_opt, param_test, param_test2, gen_lut, lut_size, lib_path, load_library,
     SBOX, INV_SBOX, mul2, mul3, mul9, mul11, mul13, mul14,
 )
 from .server import Server, sbox, many_sbox, many_wopbs_without_padding  # noqa: F401

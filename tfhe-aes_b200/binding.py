@@ -60,6 +60,20 @@ def _ctr_stream(rk_ptr, iv, first, nblk, data_ptr):
     return TfaCtrStream(rk_ptr, data_ptr, first & (2 ** 64 - 1), first >> 64, (C.c_uint8 * 16)(*iv), nblk, 0)
 
 
+class TfaCtrEncStream(C.Structure):
+    """tfa_ctr_enc_stream: one AES-CTR stream with an encrypted IV (include/tfhe_aes_b200.h)."""
+    _fields_ = [("round_keys", C.c_void_p), ("iv_ct", C.c_void_p), ("data", C.c_void_p), ("first_lo", C.c_uint64),
+                ("first_hi", C.c_uint64), ("nblk", C.c_int32), ("_pad", C.c_int32)]
+
+
+assert C.sizeof(TfaCtrEncStream) == 48
+
+
+def _ctr_enc_stream(rk_ptr, iv_ptr, first, nblk, data_ptr):
+    first %= 2 ** 128
+    return TfaCtrEncStream(rk_ptr, iv_ptr, data_ptr, first & (2 ** 64 - 1), first >> 64, nblk, 0)
+
+
 _lib = None
 
 _SIGS = {
@@ -91,6 +105,8 @@ _SIGS = {
     "tfa_aes_ctr_dev": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p],
     "tfa_aes_ctr_public_iv": [C.c_void_p, C.POINTER(TfaCtrStream), C.c_int, C.c_int, C.c_void_p],
     "tfa_aes_ctr_public_iv_dev": [C.c_void_p, C.POINTER(TfaCtrStream), C.c_int, C.c_int, C.c_void_p],
+    "tfa_aes_ctr_streams": [C.c_void_p, C.POINTER(TfaCtrEncStream), C.c_int, C.c_int, C.c_void_p],
+    "tfa_aes_ctr_streams_dev": [C.c_void_p, C.POINTER(TfaCtrEncStream), C.c_int, C.c_int, C.c_void_p],
     "tfa_add_round_key": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
     "tfa_mix_columns": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
     "tfa_inv_mix_columns": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
@@ -299,6 +315,12 @@ class Engine:
         arr = (TfaCtrStream * len(streams))(*[_ctr_stream(rk, iv, first, nblk, data) for rk, iv, first, nblk, data in streams])
         self._ck(self.lib.tfa_aes_ctr_public_iv_dev(self.h, arr, len(streams), rounds, C.c_void_p(out_ptr) if out_ptr else None))
 
+    def aes_ctr_streams_dev(self, streams, out_ptr, rounds=10):
+        """streams: list of (round_keys device pointer, encrypted IV device pointer, first, nblk, data device pointer or None);
+        out_ptr: device [total][16][8][lw].  Streams with the same IV pointer share one IV.  Asynchronous on the context stream."""
+        arr = (TfaCtrEncStream * len(streams))(*[_ctr_enc_stream(rk, iv, first, nblk, data) for rk, iv, first, nblk, data in streams])
+        self._ck(self.lib.tfa_aes_ctr_streams_dev(self.h, arr, len(streams), rounds, C.c_void_p(out_ptr) if out_ptr else None))
+
     def aes_encrypt_dev(self, rk_ptr, st_ptr, nblk):
         self._ck(self.lib.tfa_aes_encrypt_dev(self.h, C.c_void_p(rk_ptr), C.c_void_p(st_ptr), nblk))
 
@@ -464,6 +486,39 @@ class Engine:
         out = np.zeros((total, 16, 8, self.lw), dtype=np.uint64) if 0 < total < 2 ** 27 else None
         arr = (TfaCtrStream * len(structs))(*structs)
         self._ck(self.lib.tfa_aes_ctr_public_iv(self.h, arr, len(structs), rounds, _p(out)))
+        return out
+
+    def aes_ctr_streams(self, streams, rounds=10):
+        """AES-CTR with encrypted IVs, many streams in one call.  streams: list of (round_keys [rounds+1][16][8][lw], encrypted IV
+        [16][8][lw], first, nblk, data (16 * nblk bytes) or None).  Returns [total][16][8][lw]: block b of a stream encrypts
+        AES(iv + first + b) XOR data[b], streams in order.  Each distinct round-key and IV object is uploaded once, and streams that
+        pass the same IV object share its bit bootstraps."""
+        arrays, keep = {}, []
+        byte = (8 // self.bpb) * self.lw
+        sizes = {0: (rounds + 1) * 16 * byte, 1: 16 * byte}
+        for st in streams:                 # one array per distinct object: the library uploads each pointer once
+            for i in (0, 1):
+                a = st[i]
+                if a is not None and id(a) not in arrays:
+                    arr = np.ascontiguousarray(a, dtype=np.uint64)
+                    if rounds in (10, 12, 14) and arr.size != sizes[i]:   # other rounds: TfaError from the library
+                        raise ValueError(("round keys" if i == 0 else "encrypted IV") + f" must hold {sizes[i]} words, got {arr.size}")
+                    arrays[id(a)] = arr
+        structs = []
+        for rk, iv, first, nblk, data in streams:
+            d = None
+            if data is not None:
+                d = np.frombuffer(bytes(data), dtype=np.uint8).copy()
+                if len(d) != 16 * nblk:
+                    raise ValueError("data must hold 16 bytes per block")
+                keep.append(d)
+            ptr = [_p(arrays[id(a)]) if a is not None else None for a in (rk, iv)]
+            structs.append(_ctr_enc_stream(ptr[0], ptr[1], first, nblk, _p(d)))
+        total = sum(max(int(s.nblk), 0) for s in structs)
+        # an out-of-range total is left to the library to reject (TFA_ERR_PARAM) without allocating for it
+        out = np.zeros((total, 16, 8, self.lw), dtype=np.uint64) if 0 < total < 2 ** 27 else None
+        arr = (TfaCtrEncStream * len(structs))(*structs)
+        self._ck(self.lib.tfa_aes_ctr_streams(self.h, arr, len(structs), rounds, _p(out)))
         return out
 
     def xor_clear(self, states, data: bytes):

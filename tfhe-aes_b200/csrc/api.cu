@@ -182,18 +182,18 @@ static SumEntry entry(u64 *dst, std::initializer_list<const u64 *> srcs) {
     for (auto s : srcs) e.src[e.nsrc++] = s;
     return e;
 }
-// state[b][i] += rk[i]                                                        (server.rs:278-282)
-static int lin_add_round_key(tfa_ctx *ctx, u64 *state, const u64 *rk, int nblk) {
+// the same round key for each of nblk blocks
+static std::vector<const u64 *> same_rk(const u64 *rk, int nblk) { return std::vector<const u64 *>((size_t)nblk, rk); }
+// state[b][i] += rk[b][i]                                                     (server.rs:278-282)
+static int lin_add_round_key(tfa_ctx *ctx, u64 *state, const u64 *const *rk, int nblk) {
     const size_t bw = ctx->byte_words();
     std::vector<SumEntry> v;
     for (int b = 0; b < nblk; b++) for (int i = 0; i < 16; i++) {
         u64 *s = state + ((size_t)b * 16 + i) * bw;
-        v.push_back(entry(s, {s, rk + (size_t)i * bw}));
+        v.push_back(entry(s, {s, rk[b] + (size_t)i * bw}));
     }
     return dev_lwe_sum(ctx, v, (int)bw);
 }
-// the same round key for each of nblk blocks
-static std::vector<const u64 *> same_rk(const u64 *rk, int nblk) { return std::vector<const u64 *>((size_t)nblk, rk); }
 // state[b][4c+row] = MixColumns(ShiftRows(mul))[..] (+ rk[b])                 (mix_columns.rs:4-78)
 // MIX_PICK[row][j] = which of {S,2S,3S} of shifted byte j of the column (mix_columns.rs:36-75)
 static const int MIX_PICK[4][4] = {{1, 2, 0, 0}, {0, 1, 2, 0}, {0, 0, 1, 2}, {2, 0, 0, 1}};
@@ -235,6 +235,22 @@ static int lin_permute_add(tfa_ctx *ctx, const u64 *src, u64 *dst, const u64 *rk
     }
     return dev_lwe_sum(ctx, v, (int)bw);
 }
+// final ShiftRows + AddRoundKey + XOR with clear data in one pass: out[b][i] = mul[b][sr(i)] + rk[b][i], plus the clear byte
+// data[b][i] when data[b] is non-null; mul != out
+static int lin_final_round_xor(tfa_ctx *ctx, const u64 *mul, u64 *out, const u64 *const *rk, const uint8_t *const *data, int nblk) {
+    const size_t bw = ctx->byte_words();
+    std::vector<SumXorEntry> v;
+    v.reserve((size_t)16 * nblk);
+    for (int b = 0; b < nblk; b++) for (int i = 0; i < 16; i++) {
+        SumXorEntry e{};
+        e.dst = out + ((size_t)b * 16 + i) * bw;
+        e.src[e.nsrc++] = mul + ((size_t)b * 16 + sr(i)) * bw;
+        e.src[e.nsrc++] = rk[b] + (size_t)i * bw;
+        e.clear_src = data[b] ? data[b] + i : nullptr;
+        v.push_back(e);
+    }
+    return dev_lwe_sum_xor(ctx, v);
+}
 
 // ------------------------------------------------------------------------------------------------
 // Server::aes_encrypt (server.rs:39-64), nblk states at once
@@ -254,7 +270,7 @@ static int aes_encrypt_nolock(tfa_ctx *ctx, const u64 *rk, u64 *state, int nblk,
     const size_t bw = ctx->byte_words(), rkw = 16 * bw;
     WSB(mul, u64, (size_t)nblk * 16 * 3 * bw);
     const size_t mark = ctx->ws_off;
-    RC(lin_add_round_key(ctx, state, rk, nblk));                           // server.rs:42
+    RC(lin_add_round_key(ctx, state, same_rk(rk, nblk).data(), nblk));     // server.rs:42
     for (int round = 1; round < nr; round++) {
         ctx->ws_off = mark;
         RC(aes_round_nolock(ctx, same_rk(rk + (size_t)round * rkw, nblk).data(), state, nblk, mul));
@@ -269,7 +285,7 @@ static int aes_decrypt_nolock(tfa_ctx *ctx, const u64 *rk, u64 *state, int nblk,
     WSB(mul, u64, (size_t)nblk * 16 * 4 * bw);
     WSB(tmp, u64, (size_t)nblk * 16 * bw);
     const size_t mark = ctx->ws_off;
-    RC(lin_add_round_key(ctx, state, rk + (size_t)nr * rkw, nblk));        // server.rs:70
+    RC(lin_add_round_key(ctx, state, same_rk(rk + (size_t)nr * rkw, nblk).data(), nblk));  // server.rs:70
     for (int round = nr; round >= 2; round--) {
         ctx->ws_off = mark;
         // inv_shift_rows commutes with the byte-wise S-box: S-box first, permutation fused with AddRoundKey
@@ -368,21 +384,24 @@ static int add_scalar_nolock(tfa_ctx *ctx, u64 *state, const u64 *ctr_dev, int n
 // vertical packings of all blocks; per block and stage only the carry bit (block 8 of the 9-block radix of
 // server.rs:216-222) goes through its own circuit bootstrap.  Per block 15 instead of 143 bootstraps; the outputs are the
 // same functions of the same inputs (the LUTs, the selector order and the carry chain are those of add_scalar_nolock).
-static int add_scalar_from_iv_nolock(tfa_ctx *ctx, const u64 *iv_ct, const u64 *ctr_dev, int nblk, u64 *states) {
+// Several IVs: iv_ct holds niv encrypted IVs side by side, all 128 * niv bits go through one circuit-bootstrap batch, and block b
+// starts from IV blk_iv[b] (device [nblk]; nullptr when niv = 1): its vertical packings read that IV's GGSWs.
+static int add_scalar_from_iv_nolock(tfa_ctx *ctx, const u64 *iv_ct, int niv, const int32_t *blk_iv, const u64 *ctr_dev, int nblk,
+                                     u64 *states) {
     if (nblocks_per_byte(ctx) != 8) return ctx->fail(TFA_ERR_UNSUPPORTED, "add_scalar needs 1-bit blocks (client.rs:53-54)");
     const size_t bw = ctx->byte_words();
-    const int lw = ctx->lw, np = ctx->n + 1;
+    const int lw = ctx->lw, np = ctx->n + 1, nbits_iv = 128 * niv;
     const size_t ggsw_words = (size_t)ctx->p.cbs_level * (ctx->k + 1) * ctx->gsz;
-    // (1) the 128 IV bits: extract (keyswitch), circuit bootstrap, Fourier — bit t of byte b at index 8*b + t
-    WSB(iv_bits, u64, (size_t)128 * np);
-    WSB(iv_ggsw_std, u64, (size_t)128 * ggsw_words);
-    WSB(iv_ggsw_f, double2, (size_t)128 * ggsw_words / 2);
+    // (1) the IV bits: extract (keyswitch), circuit bootstrap, Fourier — bit t of byte b of IV i at index 128*i + 8*b + t
+    WSB(iv_bits, u64, (size_t)nbits_iv * np);
+    WSB(iv_ggsw_std, u64, (size_t)nbits_iv * ggsw_words);
+    WSB(iv_ggsw_f, double2, (size_t)nbits_iv * ggsw_words / 2);
     const int delta_log = 63;
     {
         const size_t mark0 = ctx->ws_off;
-        RC(dev_extract_bits(ctx, iv_ct, 128, delta_log, 1, iv_bits));
-        RC(dev_circuit_bootstrap(ctx, iv_bits, 128, iv_ggsw_std));
-        RC(dev_fourier(ctx, iv_ggsw_std, (long)128 * ctx->p.cbs_level * (ctx->k + 1) * (ctx->k + 1), ctx->p.cbs_level, iv_ggsw_f));
+        RC(dev_extract_bits(ctx, iv_ct, nbits_iv, delta_log, 1, iv_bits));
+        RC(dev_circuit_bootstrap(ctx, iv_bits, nbits_iv, iv_ggsw_std));
+        RC(dev_fourier(ctx, iv_ggsw_std, (long)nbits_iv * ctx->p.cbs_level * (ctx->k + 1) * (ctx->k + 1), ctx->p.cbs_level, iv_ggsw_f));
         ctx->ws_off = mark0;
     }
     WSB(out9, u64, (size_t)nblk * 9 * lw);
@@ -408,7 +427,7 @@ static int add_scalar_from_iv_nolock(tfa_ctx *ctx, const u64 *iv_ct, const u64 *
         }
         // the 8 sum bits and the carry bit the reference reads back (server.rs:255-263)
         RC(dev_vertical_packing(ctx, carry_ggsw_f, nblk, nbits, luts, (size_t)9 * 512, 512, 9, 512, out9,
-                                iv_ggsw_f + (size_t)index * 8 * ggsw_words / 2, 8));
+                                iv_ggsw_f + (size_t)index * 8 * ggsw_words / 2, 8, blk_iv, (size_t)128 * ggsw_words / 2));
         std::vector<SumEntry> v;
         for (int b = 0; b < nblk; b++) for (int j = 0; j < 8; j++)
             v.push_back(entry(states + ((size_t)b * 16 + index) * bw + (size_t)j * lw, {out9 + ((size_t)b * 9 + j) * lw}));
@@ -416,8 +435,8 @@ static int add_scalar_from_iv_nolock(tfa_ctx *ctx, const u64 *iv_ct, const u64 *
     }
     return TFA_OK;
 }
-static size_t add_scalar_scratch(const tfa_ctx *ctx, int nblk) {
-    return many_wopbs_scratch(ctx, nblk, 9, 9, 512) + many_wopbs_scratch(ctx, 16, 8, 8, 512) +
+static size_t add_scalar_scratch(const tfa_ctx *ctx, int nblk, int niv = 1) {
+    return many_wopbs_scratch(ctx, nblk, 9, 9, 512) + many_wopbs_scratch(ctx, 16 * niv, 8, 8, 512) +
            (size_t)nblk * (16 * ctx->byte_words() + 20 * ctx->lw + 9 * 512) * 8 + (size_t)nblk * 32 * sizeof(SumEntry) + (1 << 20);
 }
 
@@ -473,7 +492,7 @@ static int aes_ctr_nolock(tfa_ctx *ctx, const u64 *rk, const u64 *iv_ct, u64 fir
         for (int b = 0; b < nblk; b++) CU(cudaMemcpyAsync(out + (size_t)b * sw, iv_ct, sw * 8, cudaMemcpyDeviceToDevice, ctx->stream));
         RC(add_scalar_nolock(ctx, out, d_ctr, nblk));
     } else {
-        RC(add_scalar_from_iv_nolock(ctx, iv_ct, d_ctr, nblk, out));
+        RC(add_scalar_from_iv_nolock(ctx, iv_ct, 1, nullptr, d_ctr, nblk, out));
     }
     ctx->ws_off = mark;
     return aes_encrypt_nolock(ctx, rk, out, nblk);
@@ -615,18 +634,13 @@ static int aes_ctr_public_nolock(tfa_ctx *ctx, const tfa_ctr_stream *streams, co
     // (5) final round: S-box, then ShiftRows + AddRoundKey + XOR with the clear data in one pass
     ctx->ws_off = mark;
     RC(sbox_like_dev(ctx, out, B * 16, 0, mul));
-    std::vector<SumXorEntry> v;
-    v.reserve((size_t)16 * B);
-    for (int b = 0; b < B; b++) for (int i = 0; i < 16; i++) {
+    std::vector<const uint8_t *> data((size_t)B);
+    for (int b = 0; b < B; b++) {
         const tfa_ctr_stream &st = streams[p.blk_stream[b]];
-        SumXorEntry e{};
-        e.dst = out + ((size_t)b * 16 + i) * bw;
-        e.src[e.nsrc++] = mul + ((size_t)b * 16 + sr(i)) * bw;
-        e.src[e.nsrc++] = rk_of(p.blk_stream[b], nr, i);
-        e.clear_src = st.data ? st.data + (size_t)p.blk_pos[b] * 16 + i : nullptr;
-        v.push_back(e);
+        rkb[b] = rk_of(p.blk_stream[b], nr, 0);
+        data[b] = st.data ? st.data + (size_t)p.blk_pos[b] * 16 : nullptr;
     }
-    return dev_lwe_sum_xor(ctx, v);
+    return lin_final_round_xor(ctx, mul, out, rkb.data(), data.data(), B);
 }
 extern "C" int tfa_aes_ctr_public_iv_dev(tfa_ctx *ctx, const tfa_ctr_stream *streams, int nstreams, int rounds, uint64_t *out) {
     Guard g(ctx);
@@ -637,6 +651,92 @@ extern "C" int tfa_aes_ctr_public_iv_dev(tfa_ctx *ctx, const tfa_ctr_stream *str
     if (nblocks_per_byte(ctx) != 8) return ctx->fail(TFA_ERR_UNSUPPORTED, "aes_ctr_public_iv needs 1-bit blocks (client.rs:53-54)");
     RC(ws_reserve(ctx, ctr_public_scratch(ctx, p.G, p.B)));
     return aes_ctr_public_nolock(ctx, streams, p, rounds, out);
+}
+
+// ---- AES-CTR with encrypted IVs, many streams in one call ---------------------------------------------------------
+// aes_ctr_nolock for all blocks of all streams at once: the bits of every distinct IV are circuit-bootstrapped in one batch, each
+// stage of the counter add runs over all blocks (one vertical packing per stage, each block reading the GGSWs of its own stream's
+// IV), and the rounds take the round keys of each block's stream.  128 * (distinct IVs) + (128 * Nr + 15) * B PBS.
+struct CtrEncPlan {
+    int B = 0;                          // blocks
+    std::vector<const u64 *> ivs;       // distinct iv_ct pointers, in order of first use
+    std::vector<int32_t> blk_iv;        // index into ivs of each block
+    std::vector<int> blk_stream, blk_pos;
+    std::vector<u64> ctr;               // [B][2]: first + position of each block as (lo, hi), mod 2^128
+};
+static int plan_enc_ctr(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, int nstreams, int rounds, CtrEncPlan &p) {
+    if (!streams || nstreams < 1) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_streams: nstreams must be >= 1");
+    if (rounds != 10 && rounds != 12 && rounds != 14) return ctx->fail(TFA_ERR_PARAM, "rounds must be 10, 12 or 14");
+    long long total = 0;
+    for (int s = 0; s < nstreams; s++) {
+        if (streams[s].nblk < 1 || !streams[s].round_keys || !streams[s].iv_ct)
+            return ctx->fail(TFA_ERR_PARAM, "aes_ctr_streams: every stream needs nblk >= 1, round keys and an encrypted IV");
+        total += streams[s].nblk;
+    }
+    if (total > INT_MAX / 16) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_streams: too many blocks in one call");
+    p.B = (int)total;
+    p.blk_iv.reserve(p.B); p.blk_stream.reserve(p.B); p.blk_pos.reserve(p.B); p.ctr.reserve((size_t)2 * p.B);
+    for (int s = 0; s < nstreams; s++) {
+        const tfa_ctr_enc_stream &st = streams[s];
+        const int iv = (int)(std::find(p.ivs.begin(), p.ivs.end(), st.iv_ct) - p.ivs.begin());
+        if (iv == (int)p.ivs.size()) p.ivs.push_back(st.iv_ct);
+        for (int b = 0; b < st.nblk; b++) {
+            const u64 lo = st.first_lo + (u64)b;
+            p.blk_iv.push_back(iv); p.blk_stream.push_back(s); p.blk_pos.push_back(b);
+            p.ctr.push_back(lo); p.ctr.push_back(st.first_hi + (lo < st.first_lo ? 1 : 0));
+        }
+    }
+    return TFA_OK;
+}
+static size_t ctr_streams_scratch(const tfa_ctx *ctx, int niv, int B) {
+    const size_t a = aes_scratch(ctx, B, 3), c = add_scalar_scratch(ctx, B, niv) + (size_t)niv * 16 * ctx->byte_words() * 8;
+    return std::max(a, c) + (size_t)B * (16 + 4) + 1024;
+}
+// streams[s].round_keys / data: device pointers; p.ivs: host or device pointers (copied side by side first); out [B][16][8][lw] device
+static int aes_ctr_streams_nolock(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, const CtrEncPlan &p, int nr, u64 *out) {
+    const size_t bw = ctx->byte_words(), sw = 16 * bw, rkw = 16 * bw;
+    const int B = p.B, niv = (int)p.ivs.size();
+    WSB(d_ctr, u64, p.ctr.size());
+    WSB(d_blk_iv, int32_t, (size_t)B);
+    CU(cudaMemcpyAsync(d_ctr, p.ctr.data(), p.ctr.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_blk_iv, p.blk_iv.data(), (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    const size_t mark = ctx->ws_off;
+    {
+        WSB(ivs, u64, (size_t)niv * sw);
+        for (int i = 0; i < niv; i++) CU(cudaMemcpyAsync(ivs + (size_t)i * sw, p.ivs[i], sw * 8, cudaMemcpyDefault, ctx->stream));
+        RC(add_scalar_from_iv_nolock(ctx, ivs, niv, d_blk_iv, d_ctr, B, out));
+    }
+    ctx->ws_off = mark;
+    WSB(mul, u64, (size_t)B * 16 * 3 * bw);
+    const size_t mark2 = ctx->ws_off;
+    std::vector<const u64 *> rkb((size_t)B);
+    auto round_keys = [&](int round) {
+        for (int b = 0; b < B; b++) rkb[b] = streams[p.blk_stream[b]].round_keys + (size_t)round * rkw;
+        return rkb.data();
+    };
+    RC(lin_add_round_key(ctx, out, round_keys(0), B));
+    for (int round = 1; round < nr; round++) {
+        ctx->ws_off = mark2;
+        RC(aes_round_nolock(ctx, round_keys(round), out, B, mul));
+    }
+    ctx->ws_off = mark2;
+    RC(sbox_like_dev(ctx, out, B * 16, 0, mul));
+    std::vector<const uint8_t *> data((size_t)B);
+    for (int b = 0; b < B; b++) {
+        const tfa_ctr_enc_stream &st = streams[p.blk_stream[b]];
+        data[b] = st.data ? st.data + (size_t)p.blk_pos[b] * 16 : nullptr;
+    }
+    return lin_final_round_xor(ctx, mul, out, round_keys(nr), data.data(), B);
+}
+extern "C" int tfa_aes_ctr_streams_dev(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, int nstreams, int rounds, uint64_t *out) {
+    Guard g(ctx);
+    CtrEncPlan p;
+    RC(plan_enc_ctr(ctx, streams, nstreams, rounds, p));
+    if (!out) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_streams: null output");
+    RC(require_keys(ctx));
+    if (nblocks_per_byte(ctx) != 8) return ctx->fail(TFA_ERR_UNSUPPORTED, "aes_ctr_streams needs 1-bit blocks (client.rs:53-54)");
+    RC(ws_reserve(ctx, ctr_streams_scratch(ctx, (int)p.ivs.size(), p.B)));
+    return aes_ctr_streams_nolock(ctx, streams, p, rounds, out);
 }
 
 // ---- host-pointer entry points ---------------------------------------------------------------------
@@ -847,6 +947,43 @@ extern "C" int tfa_aes_ctr_public_iv(tfa_ctx *ctx, const tfa_ctr_stream *streams
     SYNC();
     return TFA_OK;
 }
+extern "C" int tfa_aes_ctr_streams(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, int nstreams, int rounds, uint64_t *out) {
+    Guard g(ctx);
+    CtrEncPlan p;
+    RC(plan_enc_ctr(ctx, streams, nstreams, rounds, p));
+    if (!out) return ctx->fail(TFA_ERR_PARAM, "aes_ctr_streams: null output");
+    RC(require_keys(ctx));
+    if (nblocks_per_byte(ctx) != 8) return ctx->fail(TFA_ERR_UNSUPPORTED, "aes_ctr_streams needs 1-bit blocks (client.rs:53-54)");
+    const size_t bw = ctx->byte_words(), rkw = (size_t)(rounds + 1) * 16 * bw, sw = (size_t)p.B * 16 * bw;
+    std::vector<const u64 *> keys;                       // distinct round-key buffers: streams under one AES key upload it once
+    for (int s = 0; s < nstreams; s++)
+        if (std::find(keys.begin(), keys.end(), streams[s].round_keys) == keys.end()) keys.push_back(streams[s].round_keys);
+    RC(ws_reserve(ctx, ctr_streams_scratch(ctx, (int)p.ivs.size(), p.B) + (keys.size() * rkw + sw) * 8 + (size_t)p.B * 16 +
+                           256 * (keys.size() + 2)));
+    WSB(d_out, u64, sw);
+    WSB(d_data, uint8_t, (size_t)p.B * 16);
+    std::vector<u64 *> d_keys;
+    for (auto k : keys) {
+        WSB(d, u64, rkw);
+        H2D(d, k, rkw);
+        d_keys.push_back(d);
+    }
+    std::vector<tfa_ctr_enc_stream> dev(streams, streams + nstreams);
+    size_t off = 0;
+    for (int s = 0; s < nstreams; s++) {
+        dev[s].round_keys = d_keys[std::find(keys.begin(), keys.end(), streams[s].round_keys) - keys.begin()];
+        if (streams[s].data) {
+            CU(cudaMemcpyAsync(d_data + off, streams[s].data, (size_t)streams[s].nblk * 16, cudaMemcpyHostToDevice, ctx->stream));
+            dev[s].data = d_data + off;
+        }
+        off += (size_t)streams[s].nblk * 16;
+    }
+    // the distinct IVs (host pointers in p.ivs) are copied to the device once each by aes_ctr_streams_nolock
+    RC(aes_ctr_streams_nolock(ctx, dev.data(), p, rounds, d_out));
+    D2H(out, d_out, sw);
+    SYNC();
+    return TFA_OK;
+}
 // transciphering step: states ^= clear data (see the header)
 extern "C" int tfa_xor_clear_dev(tfa_ctx *ctx, uint64_t *states, const uint8_t *data_dev, int nblk) {
     Guard g(ctx);
@@ -879,7 +1016,7 @@ extern "C" int tfa_add_round_key(tfa_ctx *ctx, uint64_t *states, const uint64_t 
     RC(ws_reserve(ctx, (sw + 16 * bw) * 8 + (size_t)nblk * 16 * sizeof(SumEntry)));
     WSB(d_st, u64, sw); WSB(d_rk, u64, 16 * bw);
     H2D(d_st, states, sw); H2D(d_rk, round_key, 16 * bw);
-    RC(lin_add_round_key(ctx, d_st, d_rk, nblk));
+    RC(lin_add_round_key(ctx, d_st, same_rk(d_rk, nblk).data(), nblk));
     D2H(states, d_st, sw);
     SYNC();
     return TFA_OK;

@@ -382,8 +382,11 @@ int dev_circuit_bootstrap(tfa_ctx *ctx, const u64 *lwe_small, int count, u64 *gg
 
 // SURVEY §9.4(7).  ggsw_f [njobs][nbits][...] with bit 0 = LSB.  LUT polynomials per output:
 // lut[job*lut_job_stride + o*lut_out_stride + poly*N + j], lut_size/N polynomials each.
+// Bits 0..nshared-1 of every job come from ggsw_shared instead, offset by shared_set[job] * shared_set_stride (double2) when
+// shared_set (device, [njobs]) is given.
 int dev_vertical_packing(tfa_ctx *ctx, const double2 *ggsw_f, int njobs, int nbits, const u64 *lut, size_t lut_job_stride,
-                         size_t lut_out_stride, int nouts, int lut_size, u64 *out, const double2 *ggsw_shared, int nshared) {
+                         size_t lut_out_stride, int nouts, int lut_size, u64 *out, const double2 *ggsw_shared, int nshared,
+                         const int32_t *shared_set, size_t shared_set_stride) {
     const int npoly = lut_size / ctx->N;
     int tree = ilog2u(npoly);
     if (tree > nbits) tree = 0;
@@ -416,7 +419,7 @@ int dev_vertical_packing(tfa_ctx *ctx, const double2 *ggsw_f, int njobs, int nbi
     v.ggsw_f = ggsw_f; v.tw = ctx->tw; v.lut = lut; v.glwe_init = glwe_init; v.out = out;
     v.lut_job_stride = lut_job_stride; v.lut_out_stride = lut_out_stride;
     v.nbits = nbits; v.nrot = nbits - tree; v.nouts = nouts; v.njobs = njobs;
-    v.ggsw_shared = ggsw_shared; v.nshared = nshared;
+    v.ggsw_shared = ggsw_shared; v.nshared = nshared; v.shared_set = shared_set; v.shared_set_stride = shared_set_stride;
     int G;
     if (K == 4) G = nouts >= 3 ? 3 : (nouts == 2 ? 2 : 1);
     else G = nouts >= 8 ? 8 : (nouts >= 4 ? 4 : 1);

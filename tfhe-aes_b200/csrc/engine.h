@@ -122,7 +122,8 @@ int dev_extract_bits(tfa_ctx *ctx, const u64 *in, int count, int delta_log, int 
 int dev_circuit_bootstrap(tfa_ctx *ctx, const u64 *lwe_small, int count, u64 *ggsw_std);
 int dev_vertical_packing(tfa_ctx *ctx, const double2 *ggsw_f, int njobs, int nbits, const u64 *lut, size_t lut_job_stride,
                          size_t lut_out_stride, int nouts, int lut_size, u64 *out,
-                         const double2 *ggsw_shared = nullptr, int nshared = 0);
+                         const double2 *ggsw_shared = nullptr, int nshared = 0,
+                         const int32_t *shared_set = nullptr, size_t shared_set_stride = 0);
 int dev_many_wopbs(tfa_ctx *ctx, const u64 *ct_in, int nct, int nblocks, const u64 *lut, size_t lut_job_stride,
                    size_t lut_out_stride, int nouts, int lut_size, u64 *out);
 size_t many_wopbs_scratch(const tfa_ctx *ctx, int nct, int nblocks, int nouts, int lut_size);

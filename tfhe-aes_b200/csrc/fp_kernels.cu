@@ -81,12 +81,13 @@ __global__ void __launch_bounds__(CMUX_THREADS, 1) vp_kernel(VpArgs a) {
     __syncthreads();
     const size_t ggsw_size = (size_t)LEVELS * (K + 1) * POLY_M * (K + 1);
     const cd *ggsw_job = a.ggsw_f + (size_t)job * (a.nbits - a.nshared) * ggsw_size;
+    const cd *ggsw_shared = a.shared_set ? a.ggsw_shared + (size_t)a.shared_set[job] * a.shared_set_stride : a.ggsw_shared;
 #pragma unroll 1
     for (int t = 0; t < a.nrot; t++) {
         const int deg = (t < 31 ? (1 << t) : 0) & (2 * POLY_N - 1);
         if (tid < G) sm.rot[tid] = (2 * POLY_N - deg) & (2 * POLY_N - 1);
         __syncthreads();
-        const cd *ggsw_t = t < a.nshared ? a.ggsw_shared + (size_t)t * ggsw_size : ggsw_job + (size_t)(t - a.nshared) * ggsw_size;
+        const cd *ggsw_t = t < a.nshared ? ggsw_shared + (size_t)t * ggsw_size : ggsw_job + (size_t)(t - a.nshared) * ggsw_size;
         cmux_step<K, G, BASE_LOG, LEVELS, DIFF_ROTATE>(tid, sm, rg, ggsw_t, nullptr);
     }
     for (int g = 0; g < G; g++)

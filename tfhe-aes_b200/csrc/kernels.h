@@ -28,6 +28,8 @@ struct VpArgs {
     int nrot;                 // GGSWs consumed by the blind rotation (bits 0..nrot-1)
     const double2 *ggsw_shared;  // [nshared][level][row][col][p]: GGSWs common to all jobs (bits 0..nshared-1), or nullptr
     int nshared;              // ggsw_f then holds nbits - nshared GGSWs per job
+    const int32_t *shared_set;   // [njobs] or nullptr: job j reads its shared GGSWs at ggsw_shared + shared_set[j] * shared_set_stride
+    size_t shared_set_stride;    // in double2
     int nouts;
     int njobs;
 };

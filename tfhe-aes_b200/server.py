@@ -74,3 +74,12 @@ class Server:
         rk = np.asarray(encrypted_round_keys)
         rounds = rk.size // (16 * 8 * self.engine.lw) - 1
         return self.engine.aes_ctr_public_iv([(rk, iv, first, number_of_outputs, data)], rounds)
+
+    def aes_ctr_streams(self, requests):
+        """main.rs:55-64 for many clients at once: requests is a list of (encrypted_round_keys, encrypted_iv, first,
+        number_of_outputs, data).  Returns [sum of number_of_outputs][16][8][lw], requests in order: block b of a request encrypts
+        AES(iv + first + b) XOR data[b]; data None gives the bare keystream.  AES-128/192/256 follow from the number of round
+        keys, which all requests share."""
+        requests = list(requests)
+        rounds = np.asarray(requests[0][0]).size // (16 * 8 * self.engine.lw) - 1 if requests else 10
+        return self.engine.aes_ctr_streams(requests, rounds)
