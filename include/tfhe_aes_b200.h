@@ -73,7 +73,7 @@ int tfa_ctx_key_buffers(tfa_ctx *ctx, void **dev_ptrs /* [8] */, size_t *bytes /
 int tfa_ctx_keys_ready(tfa_ctx *ctx);
 int tfa_ctx_synchronize(tfa_ctx *ctx);
 /* per-stage GPU time of everything launched since tfa_ctx_profile(ctx, 1): stages are
- * 0 ks_decompose 1 ks_gemv 2 pbs 3 pfks_decompose 4 pfks_gemv 5 fourier 6 vp 7 cmux_tree 8 linear 9 misc */
+ * 0 ks_decompose 1 ks_gemv 2 pbs 3 pfks_decompose 4 pfks_gemv 5 fourier 6 vp 7 cmux_tree 8 linear 9 misc (the GLWE pack / unpack kernels) */
 int tfa_ctx_profile(tfa_ctx *ctx, int enable);
 int tfa_ctx_profile_report(tfa_ctx *ctx, double *ms_per_stage /* [10] */, int *launch_groups /* [10] */);
 /* PBS kernel schedule (same arithmetic, SURVEY §9.4(3)): 0 = automatic (default), 2 = warp-specialised kernel, 3 = one
@@ -172,6 +172,24 @@ typedef struct tfa_ctr_enc_stream {
 int tfa_aes_ctr_streams(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, int nstreams, int rounds, uint64_t *out);
 /* streams: host array whose round_keys, iv_ct and data are device pointers; out: device; asynchronous on the context stream */
 int tfa_aes_ctr_streams_dev(tfa_ctx *ctx, const tfa_ctr_enc_stream *streams, int nstreams, int rounds, uint64_t *out);
+/* GLWE packing: `count` LWEs under the big key (lwe [count][lw], e.g. the [nblk][16][8][lw] output of the CTR entry points, i.e.
+ * 128 * nblk LWEs) in ceil(count / N) GLWEs of 16-bit words, 1 639 times smaller at PARAM_OPT (1 280 bytes per AES block instead of
+ * 2 098 176).  Format: packed [ceil(count / N)][k+1][N] uint16_t, i.e. ceil(count / N) * (k+1) * N * 2 bytes; each GLWE is its k
+ * mask polynomials, then the body (tfhe-rs GlweCiphertext order).  LWE j is coefficient j % N of GLWE j / N; coefficients past
+ * `count` in the last GLWE hold keyswitch noise only.  A word is round(x / 2^48) mod 2^16 of the native-modulus word x; widened as
+ * (uint64_t)v << 48 it gives a native-modulus GLWE under the GLWE secret key, which a tfhe-rs client decrypts with
+ * decrypt_glwe_ciphertext (coefficient j = message of LWE j).  Packing is sum_j X^(j % N) . PFKS_k(lwe_j) with pfpksk key k, the
+ * last circuit-bootstrap key, whose output has the phase of its input at coefficient 0: no key beyond the context's.  Unpacking is sample extraction of every
+ * coefficient, with no key and no bootstrap: the LWEs are again under the big key and can go into every entry point.  The
+ * arithmetic does not depend on the message encoding.  Noise (DESIGN §3): the rounding adds a standard deviation of about 2^51.2
+ * to each unpacked LWE, far below the 2^56.4 of the rounding every PBS applies.
+ * Errors: TFA_ERR_PARAM for a NULL pointer or count outside [1, INT_MAX - N + 1]; TFA_ERR_STATE for tfa_pack_lwe[_dev] without
+ * keys (unpacking needs none).  The context stays usable. */
+int tfa_pack_lwe(tfa_ctx *ctx, const uint64_t *lwe /* [count][lw] */, int count, uint16_t *packed /* [ceil(count/N)][k+1][N] */);
+int tfa_unpack_lwe(tfa_ctx *ctx, const uint16_t *packed /* [ceil(count/N)][k+1][N] */, int count, uint64_t *lwe_out /* [count][lw] */);
+/* device pointers, asynchronous on the context stream (e.g. tfa_aes_ctr_streams_dev -> tfa_pack_lwe_dev without a host round trip) */
+int tfa_pack_lwe_dev(tfa_ctx *ctx, const uint64_t *lwe_dev, int count, uint16_t *packed_dev);
+int tfa_unpack_lwe_dev(tfa_ctx *ctx, const uint16_t *packed_dev, int count, uint64_t *lwe_out_dev);
 /* one AES round on nblk states (BASELINE config 2): 16*nblk many_sbox + ShiftRows/MixColumns + AddRoundKey */
 int tfa_aes_round(tfa_ctx *ctx, const uint64_t *round_key, uint64_t *states, int nblk);
 /* linear layers alone (server.rs:278-282, mix_columns.rs:4, inv_mix_columns.rs:4, shift_rows.rs:5, inv_shift_rows.rs:5) */

@@ -107,6 +107,10 @@ _SIGS = {
     "tfa_aes_ctr_public_iv_dev": [C.c_void_p, C.POINTER(TfaCtrStream), C.c_int, C.c_int, C.c_void_p],
     "tfa_aes_ctr_streams": [C.c_void_p, C.POINTER(TfaCtrEncStream), C.c_int, C.c_int, C.c_void_p],
     "tfa_aes_ctr_streams_dev": [C.c_void_p, C.POINTER(TfaCtrEncStream), C.c_int, C.c_int, C.c_void_p],
+    "tfa_pack_lwe": [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p],
+    "tfa_pack_lwe_dev": [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p],
+    "tfa_unpack_lwe": [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p],
+    "tfa_unpack_lwe_dev": [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p],
     "tfa_add_round_key": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
     "tfa_mix_columns": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
     "tfa_inv_mix_columns": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int],
@@ -321,6 +325,14 @@ class Engine:
         arr = (TfaCtrEncStream * len(streams))(*[_ctr_enc_stream(rk, iv, first, nblk, data) for rk, iv, first, nblk, data in streams])
         self._ck(self.lib.tfa_aes_ctr_streams_dev(self.h, arr, len(streams), rounds, C.c_void_p(out_ptr) if out_ptr else None))
 
+    def pack_lwe_dev(self, lwe_ptr, count, packed_ptr):
+        """device [count][lw] LWEs -> device uint16 [ceil(count / N)][k+1][N] (tfa_pack_lwe_dev).  Asynchronous on the context stream."""
+        self._ck(self.lib.tfa_pack_lwe_dev(self.h, C.c_void_p(lwe_ptr), count, C.c_void_p(packed_ptr)))
+
+    def unpack_lwe_dev(self, packed_ptr, count, lwe_ptr):
+        """device uint16 [ceil(count / N)][k+1][N] -> device [count][lw] LWEs (tfa_unpack_lwe_dev).  Asynchronous on the context stream."""
+        self._ck(self.lib.tfa_unpack_lwe_dev(self.h, C.c_void_p(packed_ptr), count, C.c_void_p(lwe_ptr)))
+
     def aes_encrypt_dev(self, rk_ptr, st_ptr, nblk):
         self._ck(self.lib.tfa_aes_encrypt_dev(self.h, C.c_void_p(rk_ptr), C.c_void_p(st_ptr), nblk))
 
@@ -527,6 +539,27 @@ class Engine:
         assert len(data) == 16 * len(st)
         self._ck(self.lib.tfa_xor_clear(self.h, _p(st), bytes(data), len(st)))
         return st
+
+    def packed_glwes(self, count):
+        """GLWEs that hold `count` packed LWEs: ceil(count / N)"""
+        return -(-count // self.N)
+
+    def pack_lwe(self, ct):
+        """LWEs (any shape ending in lw, e.g. [nblk][16][8][lw]) -> np.uint16 [ceil(count / N)][k+1][N]: LWE j is coefficient j % N
+        of GLWE j // N, words round(x / 2^48) mod 2^16 (include/tfhe_aes_b200.h: tfa_pack_lwe)"""
+        ct = np.ascontiguousarray(ct, dtype=np.uint64).reshape(-1, self.lw)
+        out = np.zeros((self.packed_glwes(len(ct)), self.k + 1, self.N), dtype=np.uint16)
+        self._ck(self.lib.tfa_pack_lwe(self.h, _p(ct), len(ct), _p(out)))
+        return out
+
+    def unpack_lwe(self, packed, count):
+        """np.uint16 [G][k+1][N] from pack_lwe -> the first `count` LWEs [count][lw] (sample extraction, no key needed)"""
+        packed = np.ascontiguousarray(packed, dtype=np.uint16).reshape(-1, self.k + 1, self.N)
+        if count > len(packed) * self.N:
+            raise ValueError(f"{len(packed)} GLWEs hold at most {len(packed) * self.N} LWEs, not {count}")
+        out = np.zeros((max(count, 0), self.lw), dtype=np.uint64)
+        self._ck(self.lib.tfa_unpack_lwe(self.h, _p(packed), count, _p(out)))
+        return out
 
     def add_round_key(self, states, rk):
         st = np.array(states, dtype=np.uint64).reshape(-1, 16, 8, self.lw)

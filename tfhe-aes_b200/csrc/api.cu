@@ -984,6 +984,52 @@ extern "C" int tfa_aes_ctr_streams(tfa_ctx *ctx, const tfa_ctr_enc_stream *strea
     SYNC();
     return TFA_OK;
 }
+// ---- GLWE packing of LWE ciphertexts (see the header) ---------------------------------------------------------------
+static int pack_args(tfa_ctx *ctx, const void *in, int count, const void *out, const char *what) {
+    if (!in || !out) return ctx->fail(TFA_ERR_PARAM, std::string(what) + ": null pointer");
+    // the packed batch holds ceil(count / N) * N coefficient slots, counted in int
+    if (count < 1 || count > INT_MAX - (ctx->N - 1)) return ctx->fail(TFA_ERR_PARAM, std::string(what) + ": count must be in [1, INT_MAX - N + 1]");
+    return TFA_OK;
+}
+static size_t packed_words(const tfa_ctx *ctx, int count) { return (size_t)((count + ctx->N - 1) / ctx->N) * ctx->gsz; }
+extern "C" int tfa_pack_lwe_dev(tfa_ctx *ctx, const uint64_t *lwe, int count, uint16_t *packed) {
+    Guard g(ctx);
+    RC(pack_args(ctx, lwe, count, packed, "pack_lwe"));
+    RC(require_keys(ctx));
+    RC(ws_reserve(ctx, pack_lwe_scratch(ctx, count)));
+    return dev_pack_lwe(ctx, lwe, count, packed);
+}
+extern "C" int tfa_pack_lwe(tfa_ctx *ctx, const uint64_t *lwe, int count, uint16_t *packed) {
+    Guard g(ctx);
+    RC(pack_args(ctx, lwe, count, packed, "pack_lwe"));
+    RC(require_keys(ctx));
+    const size_t iw = (size_t)count * ctx->lw, pw = packed_words(ctx, count);
+    RC(ws_reserve(ctx, pack_lwe_scratch(ctx, count) + iw * 8 + pw * 2 + 512));
+    WSB(d_in, u64, iw); WSB(d_packed, uint16_t, pw);
+    H2D(d_in, lwe, iw);
+    RC(dev_pack_lwe(ctx, d_in, count, d_packed));
+    CU(cudaMemcpyAsync(packed, d_packed, pw * 2, cudaMemcpyDeviceToHost, ctx->stream));
+    SYNC();
+    return TFA_OK;
+}
+extern "C" int tfa_unpack_lwe_dev(tfa_ctx *ctx, const uint16_t *packed, int count, uint64_t *lwe_out) {
+    Guard g(ctx);
+    RC(pack_args(ctx, packed, count, lwe_out, "unpack_lwe"));
+    return dev_unpack_lwe(ctx, packed, count, lwe_out);
+}
+extern "C" int tfa_unpack_lwe(tfa_ctx *ctx, const uint16_t *packed, int count, uint64_t *lwe_out) {
+    Guard g(ctx);
+    RC(pack_args(ctx, packed, count, lwe_out, "unpack_lwe"));
+    const size_t ow = (size_t)count * ctx->lw, pw = packed_words(ctx, count);
+    RC(ws_reserve(ctx, ow * 8 + pw * 2 + 512));
+    WSB(d_packed, uint16_t, pw); WSB(d_out, u64, ow);
+    CU(cudaMemcpyAsync(d_packed, packed, pw * 2, cudaMemcpyHostToDevice, ctx->stream));
+    RC(dev_unpack_lwe(ctx, d_packed, count, d_out));
+    D2H(lwe_out, d_out, ow);
+    SYNC();
+    return TFA_OK;
+}
+
 // transciphering step: states ^= clear data (see the header)
 extern "C" int tfa_xor_clear_dev(tfa_ctx *ctx, uint64_t *states, const uint8_t *data_dev, int nblk) {
     Guard g(ctx);
@@ -1120,7 +1166,7 @@ extern "C" int tfa_pfks(tfa_ctx *ctx, int key_index, const uint64_t *in, int cou
     RC(ws_reserve(ctx, (iw + ow) * 8 + (size_t)count * (ctx->big + 1) * ctx->p.pfks_level * 2));
     WSB(d_in, u64, iw); WSB(d_out, u64, ow);
     H2D(d_in, in, iw);
-    RC(dev_pfks(ctx, d_in, count, d_out, kp1 * ctx->gsz));
+    RC(dev_pfks(ctx, d_in, count, d_out, kp1 * ctx->gsz, 0, kp1));
     CU(cudaMemcpy2DAsync(out, (size_t)ctx->gsz * 8, d_out + (size_t)key_index * ctx->gsz, (size_t)kp1 * ctx->gsz * 8, (size_t)ctx->gsz * 8,
                          count, cudaMemcpyDeviceToHost, ctx->stream));
     SYNC();

@@ -1,6 +1,7 @@
 // engine.cu — context, key preparation and the device-level stages of one WoPBS pass
 // (keyswitch -> PBS -> PFKS -> Fourier GGSW -> vertical packing), i.e. the GPU restatement of
 // many_wopbs_without_padding (many_wopbs.rs:31-116) batched over many encrypted bytes.
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 #include "engine.h"
@@ -261,9 +262,10 @@ int dev_keyswitch(tfa_ctx *ctx, const u64 *in, int count, u64 *out) {
     return TFA_OK;
 }
 
-// SURVEY §9.4(5): for every key r: glwe_r = - sum_j sum_l d_{j,l} PFPKSK_r[j][l]; out[b][r][gsz] with stride
-int dev_pfks(tfa_ctx *ctx, const u64 *in, int count, u64 *out, int out_stride) {
-    const int kp1 = ctx->k + 1, rows_pad = ctx->pf_kchunks() * 32;
+// SURVEY §9.4(5): for keys r = key0 .. key0 + nkeys - 1: glwe_r = - sum_j sum_l d_{j,l} PFPKSK_r[j][l]; out[b][r - key0][gsz] with
+// stride.  The circuit bootstrap uses all k + 1 keys, GLWE packing key k alone.
+int dev_pfks(tfa_ctx *ctx, const u64 *in, int count, u64 *out, int out_stride, int key0, int nkeys) {
+    const int rows_pad = ctx->pf_kchunks() * 32;
     const int limbs = ctx->p.pfks_base_log > 6 ? 2 : 1;
     WS(dl, int8_t, (size_t)count * rows_pad);
     int8_t *dh = nullptr;
@@ -285,16 +287,16 @@ int dev_pfks(tfa_ctx *ctx, const u64 *in, int count, u64 *out, int out_stride) {
         const int slice = (((count + nslices - 1) / nslices) + 127) & ~127;
         for (int b0 = 0; b0 < count; b0 += slice) {
             const int nb = count - b0 < slice ? count - b0 : slice;
-            CU(launch_tc5_pfks(dl + (size_t)b0 * rows_pad, dh + (size_t)b0 * rows_pad, rows_pad, ctx->pfpksk, kp1, ctx->pf_rows(), ctx->gsz, nb,
-                               out + (size_t)b0 * out_stride, out_stride, ctx->stream));
+            CU(launch_tc5_pfks(dl + (size_t)b0 * rows_pad, dh + (size_t)b0 * rows_pad, rows_pad, ctx->pfpksk + (size_t)key0 * ctx->pf_rows() * ctx->gsz,
+                               nkeys, ctx->pf_rows(), ctx->gsz, nb, out + (size_t)b0 * out_stride, out_stride, ctx->stream));
             ctx->launches += 1;
         }
         return TFA_OK;
     }
-    CU(launch_gemv_init(out, out_stride, kp1 * ctx->gsz, count, nullptr, 0, nullptr, 0, 0, 0, ctx->stream));
+    CU(launch_gemv_init(out, out_stride, nkeys * ctx->gsz, count, nullptr, 0, nullptr, 0, 0, 0, ctx->stream));
     ImmaGemvArgs g{};
-    g.dl = dl; g.dh = dh; g.kp = ctx->kp_pfpksk; g.out = out; g.out_stride = out_stride; g.rows_pad = rows_pad;
-    g.kchunks = ctx->pf_kchunks(); g.ntiles = ctx->pf_ntiles(); g.ncols = ctx->gsz; g.nkeys = kp1; g.count = count;
+    g.dl = dl; g.dh = dh; g.kp = ctx->kp_pfpksk + (size_t)key0 * ctx->pf_ntiles() * ctx->pf_kchunks() * 2048; g.out = out; g.out_stride = out_stride;
+    g.rows_pad = rows_pad; g.kchunks = ctx->pf_kchunks(); g.ntiles = ctx->pf_ntiles(); g.ncols = ctx->gsz; g.nkeys = nkeys; g.count = count;
     CU(launch_imma_gemv(g, limbs, ctx->stream));
     ctx->launches += 3;
     return TFA_OK;
@@ -375,7 +377,7 @@ int dev_circuit_bootstrap(tfa_ctx *ctx, const u64 *lwe_small, int count, u64 *gg
         ctx->launches++;
         // homomorphic_shift_boolean with DeltaLog(63): multiply by 2^(64-63-1) = 1, add q/4, PBS, add alpha
         RC(dev_pbs(ctx, lwe_small, count, l, 1, 1ull << 62, alpha, bs));
-        RC(dev_pfks(ctx, bs, count, ggsw_std + (size_t)(lvl - 1) * kp1 * ctx->gsz, L * kp1 * ctx->gsz));
+        RC(dev_pfks(ctx, bs, count, ggsw_std + (size_t)(lvl - 1) * kp1 * ctx->gsz, L * kp1 * ctx->gsz, 0, kp1));
     }
     return TFA_OK;
 }
@@ -463,6 +465,34 @@ int dev_many_wopbs(tfa_ctx *ctx, const u64 *ct_in, int nct, int nblocks, const u
     RC(dev_fourier(ctx, ggsw_std, (long)nb * ctx->p.cbs_level * (ctx->k + 1) * (ctx->k + 1), ctx->p.cbs_level, ggsw_f));
     // (3) one vertical packing per LUT output (many_wopbs.rs:267-279)
     return dev_vertical_packing(ctx, ggsw_f, nct, nbits, lut, lut_job_stride, lut_out_stride, nouts, lut_size, out);
+}
+
+// GLWE packing (DESIGN §3): PFKS with key k of the inputs of PACK_SLICE_GLWES GLWEs at a time (6 144 bits: one tcgen05 PFKS
+// launch, 126 MB of PFKS output at PARAM_OPT), then the rotation-sum and 16-bit rounding of glwe_pack_kernel.
+static const int PACK_SLICE_GLWES = 12;
+size_t pack_lwe_scratch(const tfa_ctx *ctx, int count) {
+    const size_t nb = (size_t)std::min(count, PACK_SLICE_GLWES * ctx->N);
+    return nb * ctx->gsz * 8 + nb * ctx->pf_kchunks() * 32 * 2 + 4096;   // PFKS output, two digit-limb planes
+}
+int dev_pack_lwe(tfa_ctx *ctx, const u64 *lwe, int count, uint16_t *packed) {
+    const int slice = PACK_SLICE_GLWES * ctx->N;
+    WS(pf, u64, (size_t)std::min(count, slice) * ctx->gsz);
+    const size_t mark = ctx->ws_off;
+    for (long b0 = 0; b0 < count; b0 += slice) {
+        const int nb = (int)std::min((long)count - b0, (long)slice);
+        ctx->ws_off = mark;
+        RC(dev_pfks(ctx, lwe + (size_t)b0 * ctx->lw, nb, pf, ctx->gsz, ctx->k, 1));
+        StageTimer t(ctx, ST_MISC);   // the PFKS above is timed in its own stages; the rotation-sum kernel is "misc"
+        CU(launch_glwe_pack(pf, nb, ctx->k, packed + (size_t)(b0 / ctx->N) * ctx->gsz, ctx->stream));
+        ctx->launches++;
+    }
+    return TFA_OK;
+}
+int dev_unpack_lwe(tfa_ctx *ctx, const uint16_t *packed, int count, u64 *lwe_out) {
+    StageTimer t(ctx, ST_MISC);
+    CU(launch_glwe_unpack(packed, count, ctx->k, lwe_out, ctx->stream));
+    ctx->launches++;
+    return TFA_OK;
 }
 
 // pinned staging for `bytes` of host data that an asynchronous copy on ctx->stream will read

@@ -116,7 +116,7 @@ static inline T *ws_get(tfa_ctx *ctx, size_t count) { return reinterpret_cast<T 
 // device-level stages (all asynchronous on ctx->stream, scratch from the workspace)
 int dev_keyswitch(tfa_ctx *ctx, const u64 *in, int count, u64 *out);
 int dev_pbs(tfa_ctx *ctx, const u64 *in, int count, const u64 *lut, u64 in_scale, u64 pre_add, u64 post_add, u64 *out);
-int dev_pfks(tfa_ctx *ctx, const u64 *in, int count, u64 *out, int out_stride);
+int dev_pfks(tfa_ctx *ctx, const u64 *in, int count, u64 *out, int out_stride, int key0, int nkeys);  // keys key0 .. key0 + nkeys - 1
 int dev_fourier(tfa_ctx *ctx, const u64 *polys, long npoly, int levels, double2 *out);
 int dev_extract_bits(tfa_ctx *ctx, const u64 *in, int count, int delta_log, int nbits, u64 *out /* [count][nbits][n+1], 0 = LSB */);
 int dev_circuit_bootstrap(tfa_ctx *ctx, const u64 *lwe_small, int count, u64 *ggsw_std);
@@ -127,6 +127,10 @@ int dev_vertical_packing(tfa_ctx *ctx, const double2 *ggsw_f, int njobs, int nbi
 int dev_many_wopbs(tfa_ctx *ctx, const u64 *ct_in, int nct, int nblocks, const u64 *lut, size_t lut_job_stride,
                    size_t lut_out_stride, int nouts, int lut_size, u64 *out);
 size_t many_wopbs_scratch(const tfa_ctx *ctx, int nct, int nblocks, int nouts, int lut_size);
+// GLWE packing (tfa_pack_lwe): lwe [count][lw] -> packed [ceil(count / N)][k+1][N] u16; unpack: the inverse sample extraction
+int dev_pack_lwe(tfa_ctx *ctx, const u64 *lwe, int count, uint16_t *packed);
+size_t pack_lwe_scratch(const tfa_ctx *ctx, int count);
+int dev_unpack_lwe(tfa_ctx *ctx, const uint16_t *packed, int count, u64 *lwe_out);
 int dev_lwe_sum(tfa_ctx *ctx, const std::vector<SumEntry> &entries, int unit_words);
 int dev_lwe_sum_xor(tfa_ctx *ctx, const std::vector<SumXorEntry> &entries);  // one encrypted byte per entry
 int require_keys(tfa_ctx *ctx);

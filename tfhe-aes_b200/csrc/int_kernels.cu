@@ -3,7 +3,8 @@
 //                      mix_columns.rs:4-78, inv_mix_columns.rs:4-58)
 //   lwe_sum_xor        the same plus a clear byte XORed in (public-IV CTR: counter bytes, data bytes)
 //   gemv_init          output initialisation of the keyswitch / PFKS products (imma_kernels.cu)
-//   helpers of the general extract_bits loop, CMux-tree leaves, add_scalar LUT generation.
+//   helpers of the general extract_bits loop, CMux-tree leaves, add_scalar LUT generation
+//   glwe_pack / glwe_unpack  LWEs into 16-bit GLWEs and back (tfa_pack_lwe / tfa_unpack_lwe).
 #include "kernels.h"
 
 __global__ void gemv_init_kernel(uint64_t *out, int out_stride, int total_cols, long total, const uint64_t *colsum, uint64_t offset,
@@ -135,5 +136,56 @@ __global__ void add_scalar_luts_kernel(const uint64_t *ctr, int byte_index, int 
 }
 cudaError_t launch_add_scalar_luts(const uint64_t *ctr, int nblk, int byte_index, int nbits, uint64_t *luts, cudaStream_t s) {
     add_scalar_luts_kernel<<<nblk, 256, 0, s>>>(ctr, byte_index, nbits, luts);
+    return cudaGetLastError();
+}
+
+// ---- GLWE packing of LWE ciphertexts (tfa_pack_lwe / tfa_unpack_lwe, DESIGN §3) -----------------------------------------
+// pack: packed[g][r][c] = round16( sum_i (X^i . pfks[g*512 + i])[r][c] ) over the <= 512 inputs of GLWE g.  X^i moves word j of a
+// polynomial to j + i and negates it when it wraps past 512, so coefficient c takes word (c - i) mod 512, negated when c < i.
+// round16(x) = round(x / 2^48) mod 2^16.  CTA = (128 coefficients, polynomial r, GLWE g); its 8 thread rows sum every 8th input
+// and meet in shared memory.  For a fixed input, consecutive threads read consecutive words, every word of pfks is read once, and
+// 12 GLWEs make 240 CTAs of 1 024 threads.
+#define PACK_COEFS 128
+#define PACK_ROWS 8
+__global__ void __launch_bounds__(PACK_COEFS *PACK_ROWS) glwe_pack_kernel(const uint64_t *__restrict__ pfks, int count, int kp1,
+                                                                           uint16_t *__restrict__ packed) {
+    __shared__ uint64_t part[PACK_ROWS][PACK_COEFS];
+    const int g = blockIdx.z, r = blockIdx.y, c = blockIdx.x * PACK_COEFS + threadIdx.x;
+    const int ninputs = min(512, count - g * 512);
+    const size_t gsz = (size_t)kp1 * 512;
+    const uint64_t *src = pfks + (size_t)g * 512 * gsz + (size_t)r * 512;
+    uint64_t s = 0;
+#pragma unroll 4
+    for (int i = threadIdx.y; i < ninputs; i += PACK_ROWS) {
+        const uint64_t v = src[(size_t)i * gsz + ((c - i) & 511)];
+        s += c >= i ? v : (uint64_t)0 - v;
+    }
+    part[threadIdx.y][threadIdx.x] = s;
+    __syncthreads();
+    if (threadIdx.y != 0) return;
+#pragma unroll
+    for (int t = 1; t < PACK_ROWS; t++) s += part[t][threadIdx.x];
+    packed[((size_t)g * kp1 + r) * 512 + c] = (uint16_t)(((s >> 47) + 1) >> 1);
+}
+cudaError_t launch_glwe_pack(const uint64_t *pfks, int count, int glwe_dim, uint16_t *packed, cudaStream_t s) {
+    dim3 grid(512 / PACK_COEFS, glwe_dim + 1, (count + 511) / 512);
+    glwe_pack_kernel<<<grid, dim3(PACK_COEFS, PACK_ROWS), 0, s>>>(pfks, count, glwe_dim + 1, packed);
+    return cudaGetLastError();
+}
+// unpack: LWE i is the sample extraction of coefficient j = i mod 512 of GLWE i / 512 (what the PBS kernels do for j = 0), every
+// word widened as v << 48: mask word r*512 + t is A_r[j - t] for t <= j and -A_r[512 + j - t] otherwise, the body is B[j].
+// One CTA per LWE, its threads over the words.
+__global__ void glwe_unpack_kernel(const uint16_t *__restrict__ packed, int kp1, uint64_t *__restrict__ out) {
+    const int i = blockIdx.x, j = i & 511, lw = (kp1 - 1) * 512 + 1;
+    const uint16_t *glwe = packed + (size_t)(i >> 9) * kp1 * 512;
+    uint64_t *dst = out + (size_t)i * lw;
+    for (int w = threadIdx.x; w < lw; w += blockDim.x) {
+        const int r = w >> 9, t = w & 511;   // the body (w = lw - 1) is r = kp1 - 1, t = 0
+        const uint64_t v = (uint64_t)glwe[r * 512 + ((j - t) & 511)] << 48;
+        dst[w] = t <= j ? v : (uint64_t)0 - v;
+    }
+}
+cudaError_t launch_glwe_unpack(const uint16_t *packed, int count, int glwe_dim, uint64_t *out, cudaStream_t s) {
+    glwe_unpack_kernel<<<count, 256, 0, s>>>(packed, glwe_dim + 1, out);
     return cudaGetLastError();
 }

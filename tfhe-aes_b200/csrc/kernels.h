@@ -119,3 +119,8 @@ cudaError_t launch_tree_leaves(const uint64_t *lut, size_t lut_job_stride, size_
 // counter-add LUTs of Server::add_scalar (server.rs:181-248), generated on the device
 cudaError_t launch_add_scalar_luts(const uint64_t *counters_lo_hi, int nblk, int byte_index, int nbits, uint64_t *luts,
                                    cudaStream_t s);
+// packed[g][r][c] (g < ceil(count / 512)) = round(x / 2^48) mod 2^16 of x = sum_i X^i pfks[512 g + i][r][c] over the inputs of
+// GLWE g; pfks [count][(glwe_dim + 1) * 512]: the PFKS outputs under the last circuit-bootstrap key
+cudaError_t launch_glwe_pack(const uint64_t *pfks, int count, int glwe_dim, uint16_t *packed, cudaStream_t s);
+// out [count][glwe_dim * 512 + 1]: LWE i = sample extraction of coefficient i % 512 of GLWE i / 512, words widened as v << 48
+cudaError_t launch_glwe_unpack(const uint16_t *packed, int count, int glwe_dim, uint64_t *out, cudaStream_t s);
